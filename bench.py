@@ -7,10 +7,15 @@ main_nvsf.py:72), random-init field (reference initialisers), synthetic rays, on
 step.  One "step" = one frame: time-table collapse + field evaluation of 52.2 M samples +
 compositing with the intensity / raydrop heads -> depth, intensity, raydrop per ray.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU); every rank renders its own frame (rays are
 independent: no data-path collective), value = all rays / max-over-ranks device time ("weak").
+
+--dump-outputs DIR writes what the last timed step computed on rank 0 (per ray: depth.npy,
+image.npy = intensity / raydrop, and on the CUDA path weights_sum.npy; float32) so that two builds
+can be compared output for output: the field parameters, rays and frame times are seeded, so the
+same arguments give the same inputs.
 """
 import argparse
 import ctypes
@@ -165,6 +170,14 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: one float32 DIR/<name>.npy per output tensor."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy().astype(np.float32))
+
+
 def synth_frame(S, seed):
     o, d = S.lidar_rays(-1, seed=seed)
     return o, d
@@ -313,8 +326,10 @@ def run_reference(args):
         cpu_render_sample(orc, o, d, 0.5, max(n_rays // 4, 1))
     t_total = 0.0
     for k in range(args.steps):
-        dt, _, _ = cpu_render_sample(orc, o, d, (k % 60 + 2) / 63.0, n_rays)
+        dt, _, r = cpu_render_sample(orc, o, d, (k % 60 + 2) / 63.0, n_rays)
         t_total += dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"depth": r["depth"], "image": r["image"]})
     value = n_rays * args.steps / t_total
     sample = f"{n_rays} of 67980 rays x {NUM_STEPS} samples per step (strided over the frame)"
     print(json.dumps({
@@ -580,7 +595,10 @@ def main():
     ap.add_argument("--no-train", action="store_true", help="skip the train_step sub-benchmarks")
     ap.add_argument("--no-march", action="store_true", help="skip the camera occupancy-skipping render sub-benchmark")
     ap.add_argument("--train-steps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's per-ray outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -682,6 +700,8 @@ def main():
     dens_ms = float(np.mean([e[0].elapsed_time(e[1]) for e in evs]))
     comp_ms = float(np.mean([e[1].elapsed_time(e[2]) for e in evs]))
     value = world * N * args.steps / (ms_total_max * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"depth": depth, "image": image, "weights_sum": wsum})
 
     # ---- e2e: public API, pinned host rays -> device -> render -> host result, every step ----
     o_pin = torch.from_numpy(o_np)[None].pin_memory(); d_pin = torch.from_numpy(d_np)[None].pin_memory()

@@ -1,5 +1,5 @@
-"""TEST INFRASTRUCTURE.  Builds the C oracle (gcc) and, when /root/reference is
-present (build container only), the reference extensions via build_ref.sh / build_ref_chamfer.sh."""
+"""TEST INFRASTRUCTURE.  Builds the C oracle (gcc) and, when NVSF_REFERENCE names a checkout of
+the reference project, the reference extensions via build_ref.sh / build_ref_chamfer.sh."""
 import os
 import subprocess
 import sys
@@ -30,7 +30,7 @@ def build_oracle(force=False):
 
 
 def build_ref():
-    """Compile the unmodified reference extension for sm_100a (no-op off the build box)."""
+    """Compile the unmodified reference extensions for sm_100a (no-op without NVSF_REFERENCE)."""
     out = []
     for script in ("build_ref.sh", "build_ref_chamfer.sh"):
         r = subprocess.run(["bash", os.path.join(HERE, script)], capture_output=True, text=True)

@@ -2,19 +2,18 @@
 # TEST INFRASTRUCTURE — not product code.
 #
 # Compiles the UNMODIFIED reference ray-marching extension
-# (/root/reference/nvsf/nerf/raymarching/src/{raymarching.cu,bindings.cpp})
-# for sm_100a into oracle/_ref/_raymarching_ref.so.  Sources are compiled where
-# they lie; nothing is copied into this repository.  The flags are the
+# ($NVSF_REFERENCE/nvsf/nerf/raymarching/src/{raymarching.cu,bindings.cpp}, NVSF_REFERENCE = a
+# checkout of the reference project) for sm_100a into oracle/_ref/_raymarching_ref.so.  Sources
+# are compiled where they lie; nothing is copied into this repository.  The flags are the
 # reference's own setup.py flags (nvsf/nerf/raymarching/setup.py:7-13) plus an
 # explicit -gencode for B200.  The result is a torch/pybind extension that can
-# only EXECUTE on a GPU box; `-m gpu` tests use it as the live oracle when
-# present (oracle/_ref/ is git-ignored but travels with gpurun snapshots).
+# only EXECUTE on a GPU; `-m gpu` tests use it as the live oracle when
+# present (oracle/_ref/ is git-ignored).
 #
-# /root/reference exists only in the build container; on the GPU box this
-# script is a no-op and the prebuilt .so is used.
+# Without the reference sources this script is a no-op and a prebuilt .so, if any, is used.
 set -euo pipefail
 HERE="$(cd "$(dirname "${BASH_SOURCE[0]}")" && pwd)"
-SRC=/root/reference/nvsf/nerf/raymarching/src
+SRC=${NVSF_REFERENCE:-}/nvsf/nerf/raymarching/src
 OUT="$HERE/_ref"
 if [ ! -d "$SRC" ]; then
     echo "[build_ref] $SRC not present (GPU box?) - skipping"; exit 0

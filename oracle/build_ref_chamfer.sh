@@ -2,14 +2,15 @@
 # TEST INFRASTRUCTURE — not product code.
 #
 # Compiles the UNMODIFIED reference Chamfer extension
-# (/root/reference/nvsf/nerf/chamfer3D/{chamfer3D.cu,chamfer_cuda.cpp}) for sm_100a into
-# oracle/_ref/chamfer_3D_ref.so, from the sources where they lie (nothing is copied).  The reference
-# JIT-builds these two files with torch.utils.cpp_extension.load (dist_chamfer_3D.py:27-35); this is
-# the same compile with an explicit -gencode for B200.  On the GPU box (no /root/reference) the
-# script is a no-op and the prebuilt .so is used by oracle/make_golden_chamfer.py and the -m gpu tests.
+# ($NVSF_REFERENCE/nvsf/nerf/chamfer3D/{chamfer3D.cu,chamfer_cuda.cpp}, NVSF_REFERENCE = a checkout
+# of the reference project) for sm_100a into oracle/_ref/chamfer_3D_ref.so, from the sources where
+# they lie (nothing is copied).  The reference JIT-builds these two files with
+# torch.utils.cpp_extension.load (dist_chamfer_3D.py:27-35); this is the same compile with an
+# explicit -gencode for B200.  Without the reference sources the script is a no-op and a prebuilt
+# .so, if any, is used by oracle/make_golden_chamfer.py and the -m gpu tests.
 set -euo pipefail
 HERE="$(cd "$(dirname "${BASH_SOURCE[0]}")" && pwd)"
-SRC=/root/reference/nvsf/nerf/chamfer3D
+SRC=${NVSF_REFERENCE:-}/nvsf/nerf/chamfer3D
 OUT="$HERE/_ref"
 if [ ! -d "$SRC" ]; then
     echo "[build_ref_chamfer] $SRC not present (GPU box?) - skipping"; exit 0

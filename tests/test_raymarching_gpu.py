@@ -1,14 +1,18 @@
 """Parity of the sm_100a ray-marching operators (through the C ABI / Python operator module)
-against (a) the CPU oracle and (b) the reference's own extension rebuilt for sm_100a.
+against (a) the CPU oracle and (b) the reference's own extension rebuilt for sm_100a: its stored
+outputs (tests/golden/raymarching_ref_sm100a.npz) always, the live extension when oracle/_ref/ holds
+a build of it (oracle/build_ref.sh).
 
 Bar: bit-exact for sample ids/offsets/counts, positions, deltas, near/far, Morton codes and
 bitfields; 1e-5 relative for compositing against the oracle (the oracle's exp2f is not the
 GPU's ex2.approx), bit-exact against the reference extension."""
+import os
+
 import numpy as np
 import pytest
 
 import cases
-from conftest import assert_bits_equal
+from conftest import GOLDEN, assert_bits_equal
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
@@ -401,3 +405,65 @@ def test_errors_are_loud(pkg):
                                        z.data_ptr(), z.data_ptr(), z.data_ptr(), z.data_ptr(), z.data_ptr(),
                                        z.data_ptr(), 4, None)
     assert st == -2
+
+
+# ------------------------------------------------------------------ stored outputs of the reference extension
+@pytest.fixture(scope="module")
+def gold():
+    """Inputs and outputs of the reference's own extension (raymarching.cu built for sm_100a, run on a B200 by
+    oracle/make_golden_raymarching.py): the comparison with the reference that needs nothing outside the tree."""
+    return np.load(os.path.join(GOLDEN, "raymarching_ref_sm100a.npz"))
+
+
+def test_operators_match_reference_golden(pkg, gold):
+    rm = pkg.raymarching
+    g = gold
+    nears, fars = rm.near_far_from_aabb(dev(g["nf_o"]), dev(g["nf_d"]), dev(cases.S.AABB), cases.S.MIN_NEAR)
+    assert_bits_equal(host(nears), g["nf_nears"], "nears"); assert_bits_equal(host(fars), g["nf_fars"], "fars")
+    np.testing.assert_allclose(host(rm.sph_from_ray(dev(g["sph_o"]), dev(g["sph_d"]), 3.0)), g["sph_coords"],
+                               rtol=0, atol=1e-6)
+    assert_bits_equal(host(rm.morton3D(dev(g["mt_coords"]))), g["mt_indices"], "morton3D")
+    assert_bits_equal(host(rm.morton3D_invert(dev(g["mt_indices"]))), g["mt_back"], "morton3D_invert")
+    assert_bits_equal(host(rm.packbits(dev(g["pb_grid"]), 0.25)), g["pb_bits"], "packbits")
+
+
+@pytest.mark.parametrize("ci", [0, 1, 2, 3])
+def test_march_and_composite_train_match_reference_golden(pkg, gold, ci):
+    rm = pkg.raymarching
+    p = f"mt{ci}_"
+    _, N, max_steps, perturb, m = gold[p + "meta"].tolist()
+    bf = cases.bitfield(str(gold[p + "fill"]), seed=6)
+    counter = torch.zeros(2, dtype=torch.int32, device="cuda")
+    xyzs, dirs, deltas, rays = rm.march_rays_train(
+        dev(gold[p + "o"]), dev(gold[p + "d"]), BOUND, dev(bf), C, H, dev(gold[p + "nears"]), dev(gold[p + "fars"]),
+        counter, -1, bool(perturb), -1, True, float(gold[p + "dt_gamma"]), max_steps, dev(gold[p + "noises"]))
+    assert host(counter).tolist() == [m, N]
+    assert_bits_equal(host(rays), gold[p + "rays"], "rays (canonical order)")
+    assert_bits_equal(host(xyzs), gold[p + "xyzs"], "xyzs"); assert_bits_equal(host(deltas), gold[p + "deltas"], "deltas")
+    sig, rgb = cases.field_values(m, seed=int(gold[p + "sig_seed"])); sig *= np.float32(30.0)
+    sig_t = dev(sig).requires_grad_(True); rgb_t = dev(rgb).requires_grad_(True)
+    ws, depth, image = rm.composite_rays_train(sig_t, rgb_t, deltas, rays, 1e-4)
+    assert_bits_equal(host(ws), gold[p + "ws"], "weights_sum"); assert_bits_equal(host(depth), gold[p + "depth"], "depth")
+    assert_bits_equal(host(image), gold[p + "image"], "image")
+    ((ws * dev(gold[p + "g_ws"])).sum() + (image * dev(gold[p + "g_im"])).sum()).backward()
+    assert_bits_equal(host(sig_t.grad), gold[p + "grad_sigmas"], "grad_sigmas")
+    assert_bits_equal(host(rgb_t.grad), gold[p + "grad_rgbs"], "grad_rgbs")
+
+
+def test_inference_step_matches_reference_golden(pkg, gold):
+    rm = pkg.raymarching
+    g = gold
+    n_alive, n_step = g["inf_meta"].tolist()
+    bf = cases.bitfield("shell", seed=6)
+    x, d, l = rm.march_rays(n_alive, n_step, dev(g["inf_alive"]), dev(g["inf_rays_t"]), dev(g["inf_o"]), dev(g["inf_d"]),
+                            BOUND, dev(bf), C, H, dev(g["inf_nears"]), dev(g["inf_fars"]), -1, True, cases.S.DT_GAMMA,
+                            1024, dev(g["inf_noises"]))
+    assert_bits_equal(host(x), g["inf_xyzs"], "xyzs"); assert_bits_equal(host(d), g["inf_dirs"], "dirs")
+    assert_bits_equal(host(l), g["inf_deltas"], "deltas")
+    sig, rgb = cases.field_values(n_alive * n_step, seed=71); sig *= np.float32(60.0)
+    alive, rays_t = dev(g["inf_alive"]), dev(g["inf_rays_t"])
+    ws, depth, image = dev(g["inf_ws0"]), dev(g["inf_de0"]), dev(g["inf_im0"])
+    rm.composite_rays(n_alive, n_step, alive, rays_t, dev(sig), dev(rgb), l, ws, depth, image, 1e-2)
+    assert np.array_equal(host(alive), g["inf_alive_out"])
+    assert_bits_equal(host(rays_t), g["inf_t_out"], "rays_t"); assert_bits_equal(host(ws), g["inf_ws"], "weights_sum")
+    assert_bits_equal(host(depth), g["inf_depth"], "depth"); assert_bits_equal(host(image), g["inf_image"], "image")

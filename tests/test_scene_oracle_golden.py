@@ -25,7 +25,7 @@ def SO():
 
 def test_lidar_rays_full_frame(gold, SO):
     o, d = SO.get_lidar_rays(gold["pose_a"], gold["lidar_K"], gold["lidar_K_hoz"], 66, 1030)
-    np.testing.assert_allclose(d, gold["lidar_full_a_d"], rtol=0, atol=ATOL)
+    np.testing.assert_allclose(d[gold["lidar_full_a_inds"]], gold["lidar_full_a_d"], rtol=0, atol=ATOL)
     assert np.array_equal(o[0], gold["pose_a"][:3, 3]) and (o == o[0]).all()
 
 
