@@ -33,7 +33,7 @@ extern "C" {
 #define NVSF_E_WORKSPACE (-2) /* workspace too small */
 
 /* ABI version of this header; bumped on any signature change. */
-#define NVSF_B200_ABI_VERSION 12
+#define NVSF_B200_ABI_VERSION 13
 int nvsf_abi_version(void);
 /* Human-readable text for a status returned by any nvsf_* call. */
 const char* nvsf_status_string(int status);
@@ -401,6 +401,14 @@ int nvsf_adam_begin(float* state, const float* found_inf, float beta1, float bet
 int nvsf_adam_step_guarded(float* params, const float* grads, float* exp_avg, float* exp_avg_sq,
                            size_t n, float lr, float beta1, float beta2, float eps, const float* state,
                            float grad_scale, void* stream);
+
+/* Exponential moving average of the parameters over one flat fp32 segment, replacing the reference's
+ * torch_ema.ExponentialMovingAverage.update() (trainer.py:112-114):
+ *   shadow[i] = shadow[i] - (shadow[i] - params[i]) * one_minus_decay
+ * with every operation rounded on its own (no FMA), bit-identical to torch_ema's tensor ops.  The caller
+ * computes one_minus_decay = float(1 - min(decay, (1 + t) / (10 + t))) for update number t as torch_ema
+ * does.  n a multiple of 4, 16-byte aligned pointers. */
+int nvsf_ema_update(float* shadow, const float* params, size_t n, float one_minus_decay, void* stream);
 
 /* ------------------------------------------------------------------------- */
 /* Part 4 — callers either side of the marcher: ray generation, occupancy grid  */

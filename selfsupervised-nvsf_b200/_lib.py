@@ -91,6 +91,7 @@ PROTOTYPES = {
     "nvsf_grad_found_inf": (_int, [_p, _sz, _p, _p]),
     "nvsf_adam_begin": (_int, [_p, _p, _f32, _f32, _p]),
     "nvsf_adam_step_guarded": (_int, [_p, _p, _p, _p, _sz, _f32, _f32, _f32, _f32, _p, _f32, _p]),
+    "nvsf_ema_update": (_int, [_p, _p, _sz, _f32, _p]),
     "nvsf_field_color": (_int, [_p, _p, _u32, _p, _p, _u32, _u32, _p, _u32, _p, _u32, _p]),
     # Part 4 — ray generation, occupancy grid, alive-list compaction
     "nvsf_get_lidar_rays": (_int, [_p, _p, _u32, _u32, _u32, _f32, _f32, _f32, _p, _p, _p]),
@@ -143,7 +144,7 @@ def lib():
     return _lib
 
 
-ABI_VERSION = 12
+ABI_VERSION = 13
 
 
 def check(status, what=""):

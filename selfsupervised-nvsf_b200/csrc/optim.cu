@@ -87,6 +87,23 @@ k_nonfinite(const float4* __restrict__ g, size_t n4, float* __restrict__ found) 
     if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) *found = 1.0f;
 }
 
+// EMA of the parameters (torch_ema.ExponentialMovingAverage.update, reference trainer.py:112-114):
+// s -= (s - p) * omd, rounded after every operation like torch_ema's three tensor ops
+// (tmp = s - p; tmp.mul_(omd); s.sub_(tmp)); the _rn intrinsics keep the compiler from contracting
+// the product and the subtraction into an FMA, so the shadow stays bit-identical to torch_ema's.
+__global__ void __launch_bounds__(256)
+k_ema(float4* __restrict__ s, const float4* __restrict__ p, size_t n4, float omd) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
+         i += (size_t)gridDim.x * blockDim.x) {
+        float4 si = s[i];
+        const float4 pi = __ldg(p + i);
+#define NVSF_EMA1(c) si.c = __fsub_rn(si.c, __fmul_rn(__fsub_rn(si.c, pi.c), omd));
+        NVSF_EMA1(x) NVSF_EMA1(y) NVSF_EMA1(z) NVSF_EMA1(w)
+#undef NVSF_EMA1
+        s[i] = si;
+    }
+}
+
 __global__ void k_adam_tail(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                             float* __restrict__ v, size_t begin, size_t n, float step_size, float beta1,
                             float beta2, float eps, float inv_sqrt_bc2, float grad_scale) {
@@ -133,6 +150,15 @@ extern "C" int nvsf_adam_step_guarded(float* params, const float* grads, float* 
         reinterpret_cast<float4*>(params), reinterpret_cast<const float4*>(grads),
         reinterpret_cast<float4*>(exp_avg), reinterpret_cast<float4*>(exp_avg_sq), n / 4, lr, beta1, beta2,
         eps, state, grad_scale);
+    return nvsf_launch_status();
+}
+
+extern "C" int nvsf_ema_update(float* shadow, const float* params, size_t n, float one_minus_decay, void* stream) {
+    if (n == 0) return NVSF_OK;
+    if (!shadow || !params || (n & 3) != 0) return NVSF_E_INVALID;
+    if ((((uintptr_t)shadow | (uintptr_t)params) & 15) != 0) return NVSF_E_INVALID;
+    k_ema<<<adam_blocks(n / 4), 256, 0, (cudaStream_t)stream>>>(
+        reinterpret_cast<float4*>(shadow), reinterpret_cast<const float4*>(params), n / 4, one_minus_decay);
     return nvsf_launch_status();
 }
 

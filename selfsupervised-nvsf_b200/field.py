@@ -485,6 +485,34 @@ class NeRFNetwork(nn.Module):
                 g(["flow_grid", "flow_mlp"], 0.1), g(["sigma_net"], 1.0), g(["intensity_net"], 0.1),
                 g(["raydrop_net"], 0.1), g(["color_net"], 1.0)]
 
+    def reference_param_groups(self):
+        """The reference optimiser's 11 parameter groups (network_dynamic.py:335-357) as
+        [{"params": [reference key, ...], "lr": lr factor}]: get_params' groups under the reference's
+        checkpoint keys, plus the groups of the zero-size tcnn view encodings after the four encoder
+        groups.  Pinned by tests/golden/state_dict_manifest.json ("optimizer_groups")."""
+        name_of = {id(p): n for n, p in self.named_parameters()}
+        keys_of = {}
+        for key, name, _, _, _ in self._reference_keys():
+            keys_of.setdefault(name, []).append(key)
+        groups = [{"params": [k for p in g["params"] for k in keys_of[name_of[id(p)]]], "lr": g["lr"]}
+                  for g in self.get_params(1.0)]
+        groups[4:4] = [{"params": [f"view_encoder_{m}.params"], "lr": 1.0} for m in ("lidar", "camera")]
+        return groups
+
+    def reference_parameters(self):
+        """[(reference key, shape)] of every parameter of the reference model in its `model.parameters()`
+        order (the order of torch_ema's shadow_params): the state_dict keys without the aabb buffers.
+        Besides the hot-path keys of _reference_keys this lists the un-suffixed planes_encoder /
+        hash_encoder (shaped like the _lidar ones) and the (0,) view encodings, which the reference
+        constructs but never reads or optimises."""
+        hot = [(k, tuple(s)) for k, _, _, _, s in self._reference_keys()]
+        pick = lambda *prefixes: [(k, s) for k, s in hot if k.startswith(prefixes)]
+        enc = lambda m: pick(f"planes_encoder_{m}.") + pick(f"hash_encoder_{m}.")
+        return ([(k.replace("_lidar.", ".", 1), s) for k, s in enc("lidar")] + enc("lidar") + enc("camera")
+                + [("view_encoder_lidar.params", (0,))]
+                + pick("flow_net.", "sigma_net.", "intensity_net.", "raydrop_net.")
+                + [("view_encoder_camera.params", (0,))] + pick("color_net."))
+
     def _params_c(self, lidar):
         m = "lidar" if lidar else "camera"
         ps = FieldParamsC()
