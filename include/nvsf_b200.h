@@ -33,7 +33,7 @@ extern "C" {
 #define NVSF_E_WORKSPACE (-2) /* workspace too small */
 
 /* ABI version of this header; bumped on any signature change. */
-#define NVSF_B200_ABI_VERSION 13
+#define NVSF_B200_ABI_VERSION 14
 int nvsf_abi_version(void);
 /* Human-readable text for a status returned by any nvsf_* call. */
 const char* nvsf_status_string(int status);
@@ -547,6 +547,65 @@ int nvsf_chamfer_forward(const float* xyz1, const float* xyz2, uint32_t b, uint3
 int nvsf_chamfer_backward(const float* xyz1, const float* xyz2, uint32_t b, uint32_t n, uint32_t m,
                           const float* grad_dist1, const float* grad_dist2, const int32_t* idx1,
                           const int32_t* idx2, float* grad_xyz1, float* grad_xyz2, void* stream);
+
+/* ------------------------------------------------------------------------- */
+/* Part 6 — evaluation of rendered frames                                     */
+/* ------------------------------------------------------------------------- */
+/* Replaces the host-side scoring of Trainer.evaluate_one_epoch / test_step (trainer.py:817-903,
+ * 1458-1846): the meters of nvsf/lib/error_matrices.py and the range image -> point cloud conversion of
+ * nvsf/lib/convert.py.  Metric definitions: DESIGN.md §3.5.  Reductions run in a fixed order, so the same
+ * inputs give a bit-identical result; nothing is read back to the host. */
+
+/* Chamfer forward with the cloud sizes in device memory: xyz1 [cap_n,3], xyz2 [cap_m,3] hold *n / *m
+ * (device int32, clamped to [0, capacity]) points followed by padding.  dist / idx of the first *n / *m rows
+ * are bit-identical to nvsf_chamfer_forward on the trimmed clouds (same arithmetic, same first minimum); rows
+ * past a count get 0 / -1, and every query gets +inf / -1 when the other cloud is empty.  workspace:
+ * nvsf_chamfer_workspace_bytes(1, cap_n, cap_m). */
+int nvsf_chamfer_forward_counted(const float* xyz1, const float* xyz2, uint32_t cap_n, uint32_t cap_m,
+                                 const int32_t* n, const int32_t* m, float* dist1, float* dist2, int32_t* idx1,
+                                 int32_t* idx2, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Range image -> point cloud (convert.py): for every pixel p = j*W + i of depth [H,W] whose masked depth
+ * depth * (raydrop > raydrop_threshold) is non-zero (raydrop [H,W] may be NULL: no mask), the row
+ * lidar_dir(i, j) * (masked depth / scale), with lidar_dir the direction of nvsf_get_lidar_rays at the
+ * identity pose; plus intensity[p] as a 4th column when intensity [H,W] is given.  points [H*W, 3 or 4]: kept
+ * pixels in row-major order, then zero rows; *count (device int32) = number kept.  Order-preserving prefix sums,
+ * no atomics.  H*W <= 2^26. */
+size_t nvsf_lidar_points_workspace_bytes(uint32_t H, uint32_t W);
+int nvsf_lidar_points(const float* depth, const float* raydrop, float raydrop_threshold, const float* intensity,
+                      uint32_t H, uint32_t W, float fov_up, float fov, float fov_hoz, float scale, float* points,
+                      int32_t* count, void* workspace, size_t workspace_bytes, void* stream);
+
+/* One LiDAR frame's metric row (NVSF_EVAL_LIDAR_K floats, column order below).  depth [H,W] and image [H,W,2]
+ * (raydrop probability, intensity) are render_frame's outputs; gt [H,W,3] = (raydrop mask, intensity, depth)
+ * as for nvsf_loss_lidar.  workspace (16-byte aligned): nvsf_eval_lidar_workspace_bytes(H, W). */
+#define NVSF_EVAL_LIDAR_K 15
+#define NVSF_EVAL_DEPTH_RMSE 0
+#define NVSF_EVAL_DEPTH_MEDAE 1
+#define NVSF_EVAL_DEPTH_PSNR 2
+#define NVSF_EVAL_DEPTH_SSIM 3
+#define NVSF_EVAL_INTENSITY_RMSE 4
+#define NVSF_EVAL_INTENSITY_MEDAE 5
+#define NVSF_EVAL_INTENSITY_PSNR 6
+#define NVSF_EVAL_INTENSITY_SSIM 7
+#define NVSF_EVAL_RAYDROP_RMSE 8
+#define NVSF_EVAL_RAYDROP_ACC 9
+#define NVSF_EVAL_RAYDROP_F1 10
+#define NVSF_EVAL_CHAMFER 11
+#define NVSF_EVAL_FSCORE 12
+#define NVSF_EVAL_POINTS_PRED 13
+#define NVSF_EVAL_POINTS_GT 14
+size_t nvsf_eval_lidar_workspace_bytes(uint32_t H, uint32_t W);
+int nvsf_eval_lidar(const float* depth, const float* image, const float* gt, uint32_t H, uint32_t W, float fov_up,
+                    float fov, float fov_hoz, float scale, float max_depth, float fscore_threshold, float* row,
+                    void* workspace, size_t workspace_bytes, void* stream);
+
+/* One camera frame's row (PSNR, SSIM) of pred / gt [H,W,3] in [0,1]: PSNR = -10 log10(MSE), SSIM = mean of
+ * the per-channel SSIMs with data range 1.  workspace (16-byte aligned): nvsf_eval_camera_workspace_bytes. */
+#define NVSF_EVAL_CAMERA_K 2
+size_t nvsf_eval_camera_workspace_bytes(uint32_t H, uint32_t W);
+int nvsf_eval_camera(const float* pred, const float* gt, uint32_t H, uint32_t W, float* row, void* workspace,
+                     size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

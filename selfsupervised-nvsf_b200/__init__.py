@@ -12,6 +12,7 @@ Sub-modules
     optim         Adam over the flat parameter / gradient buffers (CUDA kernel)
     losses        lidar_loss / rgb_loss of the reference's train_step, loss + derivative in one kernel
     chamfer       drop-in for reference ``nvsf.nerf.chamfer3D.dist_chamfer_3D`` (chamfer_3DDist)
+    metrics       evaluation on the device: lidar_points (range image -> point cloud), LidarMeter / CameraMeter
     _lib          ctypes binding of the C ABI (include/nvsf_b200.h)
     build         compiles csrc/*.cu into libnvsf_b200.so with nvcc (sm_100a)
 """
@@ -23,6 +24,7 @@ from . import dist  # noqa: F401
 from . import optim  # noqa: F401
 from . import losses  # noqa: F401
 from . import chamfer  # noqa: F401
+from . import metrics  # noqa: F401
 from .field import NeRFNetwork  # noqa: F401
 
 __version__ = "0.1.0"

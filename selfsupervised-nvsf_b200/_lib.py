@@ -112,6 +112,14 @@ PROTOTYPES = {
     "nvsf_chamfer_workspace_bytes": (_sz, [_u32, _u32, _u32]),
     "nvsf_chamfer_forward": (_int, [_p, _p, _u32, _u32, _u32, _p, _p, _p, _p, _p, _sz, _p]),
     "nvsf_chamfer_backward": (_int, [_p, _p, _u32, _u32, _u32, _p, _p, _p, _p, _p, _p, _p]),
+    # Part 6 — evaluation
+    "nvsf_chamfer_forward_counted": (_int, [_p, _p, _u32, _u32, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    "nvsf_lidar_points_workspace_bytes": (_sz, [_u32, _u32]),
+    "nvsf_lidar_points": (_int, [_p, _p, _f32, _p, _u32, _u32, _f32, _f32, _f32, _f32, _p, _p, _p, _sz, _p]),
+    "nvsf_eval_lidar_workspace_bytes": (_sz, [_u32, _u32]),
+    "nvsf_eval_lidar": (_int, [_p, _p, _p, _u32, _u32, _f32, _f32, _f32, _f32, _f32, _f32, _p, _p, _sz, _p]),
+    "nvsf_eval_camera_workspace_bytes": (_sz, [_u32, _u32]),
+    "nvsf_eval_camera": (_int, [_p, _p, _u32, _u32, _p, _p, _sz, _p]),
 }
 
 _lib = None
@@ -144,7 +152,7 @@ def lib():
     return _lib
 
 
-ABI_VERSION = 13
+ABI_VERSION = 14
 
 
 def check(status, what=""):

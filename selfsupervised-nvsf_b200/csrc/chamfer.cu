@@ -25,13 +25,16 @@ constexpr int kChThreads = 256;
 constexpr int kChQueries = 2 * kChThreads;   // per CTA
 constexpr int kChTile = 1024;                // target points per shared-memory tile
 
-__global__ void __launch_bounds__(kChThreads)
-k_chamfer_nn(const float* __restrict__ xyz, uint32_t n, const float* __restrict__ xyz2, uint32_t m,
-             uint32_t per_split, unsigned long long* __restrict__ keys) {
+// a point count kept in device memory, clamped to [0, capacity]
+__device__ __forceinline__ uint32_t device_count(const int32_t* __restrict__ c, uint32_t cap) {
+    return (uint32_t)min(max(__ldg(c), 0), (int32_t)cap);
+}
+
+// One CTA's share of the nearest-neighbour scan: queries q[blockIdx.x * kChQueries ...] against targets
+// [blockIdx.y * per_split, +per_split) of t, folded into keys[j] with atomicMin.
+__device__ __forceinline__ void chamfer_nn_tile(const float* __restrict__ q, uint32_t n, const float* __restrict__ t,
+                                                uint32_t m, uint32_t per_split, unsigned long long* __restrict__ kb) {
     __shared__ float sx[kChTile], sy[kChTile], sz[kChTile];
-    const uint32_t b = blockIdx.z;
-    const float* q = xyz + (size_t)b * n * 3;
-    const float* t = xyz2 + (size_t)b * m * 3;
     const uint32_t j0 = blockIdx.x * kChQueries + threadIdx.x, j1 = j0 + kChThreads;
     float x0 = 0.f, y0 = 0.f, z0 = 0.f, x1 = 0.f, y1 = 0.f, z1 = 0.f;
     if (j0 < n) { x0 = __ldg(q + 3 * (size_t)j0); y0 = __ldg(q + 3 * (size_t)j0 + 1); z0 = __ldg(q + 3 * (size_t)j0 + 2); }
@@ -63,10 +66,27 @@ k_chamfer_nn(const float* __restrict__ xyz, uint32_t n, const float* __restrict_
         }
     }
     if (k_begin < k_end) {
-        unsigned long long* kb = keys + (size_t)b * n;
         if (j0 < n) atomicMin(kb + j0, ((unsigned long long)__float_as_uint(best0) << 32) | bi0);
         if (j1 < n) atomicMin(kb + j1, ((unsigned long long)__float_as_uint(best1) << 32) | bi1);
     }
+}
+
+__global__ void __launch_bounds__(kChThreads)
+k_chamfer_nn(const float* __restrict__ xyz, uint32_t n, const float* __restrict__ xyz2, uint32_t m,
+             uint32_t per_split, unsigned long long* __restrict__ keys) {
+    const uint32_t b = blockIdx.z;
+    chamfer_nn_tile(xyz + (size_t)b * n * 3, n, xyz2 + (size_t)b * m * 3, m, per_split, keys + (size_t)b * n);
+}
+
+// The same scan with the cloud sizes read from device memory (clouds padded to a capacity; the grid is laid
+// out for the capacities and CTAs past the counts return at once).
+__global__ void __launch_bounds__(kChThreads)
+k_chamfer_nn_counted(const float* __restrict__ xyz, uint32_t cap_n, const int32_t* __restrict__ n_dev,
+                     const float* __restrict__ xyz2, uint32_t cap_m, const int32_t* __restrict__ m_dev,
+                     uint32_t per_split, unsigned long long* __restrict__ keys) {
+    const uint32_t n = device_count(n_dev, cap_n), m = device_count(m_dev, cap_m);
+    if (blockIdx.x * kChQueries >= n || blockIdx.y * per_split >= m) return;
+    chamfer_nn_tile(xyz, n, xyz2, m, per_split, keys);
 }
 
 // keys [c1 | c2] -> (dist1, idx1) and (dist2, idx2) in one launch
@@ -80,6 +100,32 @@ __global__ void k_chamfer_unpack(const unsigned long long* __restrict__ keys, si
     const int32_t id = (int32_t)(uint32_t)k;
     if (i < c1) { dist1[i] = d; idx1[i] = id; }
     else { dist2[i - c1] = d; idx2[i - c1] = id; }
+}
+
+// keys [cap_n | cap_m] -> dist / idx of the counted forward.  A query whose target cloud is empty keeps the
+// all-ones key and gets +inf / -1; rows past a count get 0 / -1.
+__global__ void k_chamfer_unpack_counted(const unsigned long long* __restrict__ keys, uint32_t cap_n, uint32_t cap_m,
+                                         const int32_t* __restrict__ n_dev, const int32_t* __restrict__ m_dev,
+                                         float* __restrict__ dist1, int32_t* __restrict__ idx1,
+                                         float* __restrict__ dist2, int32_t* __restrict__ idx2) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)cap_n + cap_m) return;
+    const bool first = i < cap_n;
+    const uint32_t r = first ? (uint32_t)i : (uint32_t)(i - cap_n);
+    const uint32_t cnt = first ? device_count(n_dev, cap_n) : device_count(m_dev, cap_m);
+    float d = 0.f;
+    int32_t id = -1;
+    if (r < cnt) {
+        const unsigned long long k = keys[i];
+        if (k == ~0ull) {
+            d = INFINITY;
+        } else {
+            d = __uint_as_float((uint32_t)(k >> 32));
+            id = (int32_t)(uint32_t)k;
+        }
+    }
+    if (first) { dist1[r] = d; idx1[r] = id; }
+    else { dist2[r] = d; idx2[r] = id; }
 }
 
 // chamfer3D.cu:151-178: g = 2 * grad_dist[j]; grad_a[j] += g (a_j - b_idx); grad_b[idx] -= g (a_j - b_idx)
@@ -106,8 +152,12 @@ k_chamfer_grad(const float* __restrict__ a, uint32_t n, const float* __restrict_
     }
 }
 
-void launch_nn(const float* q, uint32_t n, const float* t, uint32_t m, uint32_t b,
-               unsigned long long* keys, int sms, cudaStream_t s) {
+// grid (query blocks, target ranges) of one scan direction
+struct NnGrid {
+    uint32_t qblocks, splits, per_split;
+};
+
+NnGrid nn_grid(uint32_t n, uint32_t m, uint32_t b, int sms) {
     const uint32_t qblocks = nvsf_div_up(n, (uint32_t)kChQueries);
     // enough target ranges to put ~2 CTAs on every SM; ranges are multiples of 128 targets (the trainer's single
     // batch of 4096 x 4096 points became 8 x 4 = 32 CTAs with whole 1024-target tiles: 0.33 ms against the
@@ -116,7 +166,20 @@ void launch_nn(const float* q, uint32_t n, const float* t, uint32_t m, uint32_t 
     uint32_t splits = std::max(1u, std::min(nvsf_div_up(m, gran), (2u * (uint32_t)sms) / std::max(1u, qblocks * b)));
     const uint32_t per_split = nvsf_div_up(nvsf_div_up(m, splits), gran) * gran;
     splits = nvsf_div_up(m, per_split);
-    k_chamfer_nn<<<dim3(qblocks, splits, b), kChThreads, 0, s>>>(q, n, t, m, per_split, keys);
+    return {qblocks, splits, per_split};
+}
+
+void launch_nn(const float* q, uint32_t n, const float* t, uint32_t m, uint32_t b,
+               unsigned long long* keys, int sms, cudaStream_t s) {
+    const NnGrid g = nn_grid(n, m, b, sms);
+    k_chamfer_nn<<<dim3(g.qblocks, g.splits, b), kChThreads, 0, s>>>(q, n, t, m, g.per_split, keys);
+}
+
+int sm_count() {
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    return sms;
 }
 
 }  // namespace
@@ -135,9 +198,7 @@ int nvsf_chamfer_forward(const float* xyz1, const float* xyz2, uint32_t b, uint3
     if (!xyz1 || !xyz2 || !dist1 || !dist2 || !idx1 || !idx2 || !workspace) return NVSF_E_INVALID;
     if (workspace_bytes < nvsf_chamfer_workspace_bytes(b, n, m)) return NVSF_E_WORKSPACE;
     cudaStream_t s = (cudaStream_t)stream;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = sm_count();
     unsigned long long* k1 = reinterpret_cast<unsigned long long*>(workspace);
     unsigned long long* k2 = k1 + (size_t)b * n;
     cudaMemsetAsync(workspace, 0xff, nvsf_chamfer_workspace_bytes(b, n, m), s);
@@ -146,6 +207,27 @@ int nvsf_chamfer_forward(const float* xyz1, const float* xyz2, uint32_t b, uint3
     const size_t c1 = (size_t)b * n, c2 = (size_t)b * m;
     k_chamfer_unpack<<<(unsigned)nvsf_div_up(c1 + c2, (size_t)256), 256, 0, s>>>(k1, c1, c2, dist1, idx1, dist2,
                                                                               idx2);
+    return nvsf_launch_status();
+}
+
+int nvsf_chamfer_forward_counted(const float* xyz1, const float* xyz2, uint32_t cap_n, uint32_t cap_m,
+                                 const int32_t* n, const int32_t* m, float* dist1, float* dist2, int32_t* idx1,
+                                 int32_t* idx2, void* workspace, size_t workspace_bytes, void* stream) {
+    if (cap_n == 0 || cap_m == 0 || cap_n > INT32_MAX || cap_m > INT32_MAX) return NVSF_E_INVALID;
+    if (!xyz1 || !xyz2 || !n || !m || !dist1 || !dist2 || !idx1 || !idx2 || !workspace) return NVSF_E_INVALID;
+    if (workspace_bytes < nvsf_chamfer_workspace_bytes(1, cap_n, cap_m)) return NVSF_E_WORKSPACE;
+    cudaStream_t s = (cudaStream_t)stream;
+    const int sms = sm_count();
+    unsigned long long* k1 = reinterpret_cast<unsigned long long*>(workspace);
+    unsigned long long* k2 = k1 + cap_n;
+    cudaMemsetAsync(workspace, 0xff, nvsf_chamfer_workspace_bytes(1, cap_n, cap_m), s);
+    const NnGrid g1 = nn_grid(cap_n, cap_m, 1, sms), g2 = nn_grid(cap_m, cap_n, 1, sms);
+    k_chamfer_nn_counted<<<dim3(g1.qblocks, g1.splits), kChThreads, 0, s>>>(xyz1, cap_n, n, xyz2, cap_m, m,
+                                                                           g1.per_split, k1);
+    k_chamfer_nn_counted<<<dim3(g2.qblocks, g2.splits), kChThreads, 0, s>>>(xyz2, cap_m, m, xyz1, cap_n, n,
+                                                                           g2.per_split, k2);
+    k_chamfer_unpack_counted<<<(unsigned)nvsf_div_up((size_t)cap_n + cap_m, (size_t)256), 256, 0, s>>>(
+        k1, cap_n, cap_m, n, m, dist1, idx1, dist2, idx2);
     return nvsf_launch_status();
 }
 

@@ -14,6 +14,7 @@
 #include <algorithm>
 
 #include "common.cuh"
+#include "lidar_dir.cuh"
 
 namespace {
 
@@ -47,8 +48,7 @@ __device__ __forceinline__ void emit_ray(const Pose& P, float x, float y, float 
     }
 }
 
-// dataset_utils.py:512-530: beta = -(i - W/2)/W * fov_hoz/180*pi, alpha = (fov_up - j/H*fov)/180*pi,
-// d = (cos a cos b, cos a sin b, sin a), i = column, j = row of pixel id = j*W + i.
+// direction of pixel id p = j*W + i: lidar_dir.cuh (dataset_utils.py:512-530)
 __global__ void __launch_bounds__(256)
 k_lidar_rays(const float* __restrict__ pose, const int64_t* __restrict__ inds, uint32_t n,
              uint32_t H, uint32_t W, float fov_up, float fov, float fov_hoz,
@@ -57,16 +57,9 @@ k_lidar_rays(const float* __restrict__ pose, const int64_t* __restrict__ inds, u
     if (k >= n) return;
     const Pose P = load_pose(pose);
     const int64_t p = inds ? inds[k] : (int64_t)k;
-    const float i = (float)(p % W), j = (float)(p / W);
-    const float kPi = 3.14159265358979323846f;
-    float beta = __fdiv_rn(-(i - (float)W * 0.5f), (float)W);
-    beta = __fmul_rn(__fdiv_rn(__fmul_rn(beta, fov_hoz), 180.0f), kPi);
-    float alpha = __fsub_rn(fov_up, __fmul_rn(__fdiv_rn(j, (float)H), fov));
-    alpha = __fmul_rn(__fdiv_rn(alpha, 180.0f), kPi);
-    float sa, ca, sb, cb;
-    sincosf(alpha, &sa, &ca);
-    sincosf(beta, &sb, &cb);
-    emit_ray(P, __fmul_rn(ca, cb), __fmul_rn(ca, sb), sa, k, rays_o, rays_d);
+    float x, y, z;
+    lidar_dir(p, H, W, fov_up, fov, fov_hoz, x, y, z);
+    emit_ray(P, x, y, z, k, rays_o, rays_d);
 }
 
 // dataset_utils.py:563-681: xs = (i + 0.5 - cx)/fx, ys = (j + 0.5 - cy)/fy, zs = 1, normalised.
