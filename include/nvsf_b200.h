@@ -33,7 +33,7 @@ extern "C" {
 #define NVSF_E_WORKSPACE (-2) /* workspace too small */
 
 /* ABI version of this header; bumped on any signature change. */
-#define NVSF_B200_ABI_VERSION 14
+#define NVSF_B200_ABI_VERSION 15
 int nvsf_abi_version(void);
 /* Human-readable text for a status returned by any nvsf_* call. */
 const char* nvsf_status_string(int status);
@@ -427,6 +427,29 @@ int nvsf_get_lidar_rays(const float* pose, const int64_t* inds, uint32_t n, uint
 int nvsf_get_rays(const float* pose, const int64_t* inds, uint32_t n, uint32_t H, uint32_t W,
                   float fx, float fy, float cx, float cy, float* rays_o, float* rays_d,
                   void* stream);
+
+/* Error-map guided pixel selection: replaces the error-map branch of get_lidar_rays / get_rays
+ * (dataset/dataset_utils.py; torch-ngp's convention, parity unpinned: DESIGN.md §3.5) and the
+ * error-map update of Trainer.train_step (trainer.py:551-560), with no host round trip.
+ *
+ * nvsf_error_map_sample, for one map error_map [R = res*res] (fp32, device): N distinct coarse cells
+ *   with probability proportional to the map, without replacement (torch.multinomial's distribution):
+ *   the N smallest keys expo[i] / error_map[i] (fp32 IEEE division, ties to the lower cell), expo [R]
+ *   exponential draws (>= 0).  Cells with error_map <= 0 or non-finite have zero weight; when fewer
+ *   than N cells have positive weight all of them are taken and the rest is filled with the smallest
+ *   expo among the other cells.  inds_coarse [N] (int64) receives the cells in ascending cell order,
+ *   not in draw order; inds [N] the pixel row*W + col, row = min(trunc(fl(fl(cr*sx) + fl(u0*sx))), H-1),
+ *   col = min(trunc(fl(fl(cc*sy) + fl(u1*sy))), W-1), cr = cell / res, cc = cell % res,
+ *   sx = float(H/res), sy = float(W/res), (u0, u1) = jitter[j] ([N,2] in [0,1)) for the j-th output.
+ *   One CTA, the R keys in shared memory: res <= NVSF_ERROR_MAP_MAX_RES; 1 <= N <= R.
+ * nvsf_error_map_update, for one map row: error_map[c] = fl(fl(0.1f*error_map[c]) + fl(0.9f*loss[j]))
+ *   with c = inds_coarse[j], j < N (distinct cells, as nvsf_error_map_sample returns them); a cell
+ *   outside [0, R) is skipped. */
+#define NVSF_ERROR_MAP_MAX_RES 224
+int nvsf_error_map_sample(const float* error_map, const float* expo, const float* jitter, uint32_t res,
+                          uint32_t N, uint32_t H, uint32_t W, int64_t* inds_coarse, int64_t* inds, void* stream);
+int nvsf_error_map_update(float* error_map, uint32_t R, const int64_t* inds_coarse, uint32_t N, const float* loss,
+                          void* stream);
 
 /* Occupancy-grid maintenance producing the `density_bitfield` that march_rays_train / march_rays
  * read (raymarching.py:179,379).  The reference ships only morton3D / packbits and no update

@@ -7,7 +7,8 @@ Sub-modules
     raymarching   drop-in for reference ``nvsf.nerf.raymarching.raymarching``
     field         NeRFNetwork: density / color / flow / run / render of the reference model on the GPU
                   kernels, plus the occupancy-grid update and the march_rays* render loops (run_cuda)
-    rays          get_lidar_rays / get_rays (reference dataset_utils.py) generated on the device
+    rays          get_lidar_rays / get_rays (reference dataset_utils.py) generated on the device, error-map
+                  guided sampling and update_error_map
     dist          ray sharding + flat-buffer gradient all-reduce (one process per GPU)
     optim         Adam over the flat parameter / gradient buffers (CUDA kernel)
     losses        lidar_loss / rgb_loss of the reference's train_step, loss + derivative in one kernel

@@ -96,6 +96,8 @@ PROTOTYPES = {
     # Part 4 — ray generation, occupancy grid, alive-list compaction
     "nvsf_get_lidar_rays": (_int, [_p, _p, _u32, _u32, _u32, _f32, _f32, _f32, _p, _p, _p]),
     "nvsf_get_rays": (_int, [_p, _p, _u32, _u32, _u32, _f32, _f32, _f32, _f32, _p, _p, _p]),
+    "nvsf_error_map_sample": (_int, [_p, _p, _p, _u32, _u32, _u32, _u32, _p, _p, _p]),
+    "nvsf_error_map_update": (_int, [_p, _u32, _p, _u32, _p, _p]),
     "nvsf_grid_cell_points": (_int, [_u32, _u32, _f32, _p, _p, _p]),
     "nvsf_grid_cell_points_range": (_int, [_u32, _u32, _f32, _p, ctypes.c_uint64, ctypes.c_uint64, _p, _p]),
     "nvsf_grid_accumulate": (_int, [_p, _p, _u32, _f32, _u32, _p]),
@@ -152,7 +154,7 @@ def lib():
     return _lib
 
 
-ABI_VERSION = 14
+ABI_VERSION = 15
 
 
 def check(status, what=""):

@@ -10,6 +10,7 @@
 
 #include "common.cuh"
 #include "lidar_dir.cuh"
+#include "radix_select.cuh"
 
 namespace {
 
@@ -277,34 +278,12 @@ constexpr int kSelBlock = 1024;
 __global__ void __launch_bounds__(kSelBlock)
 k_select(const float* __restrict__ arrays, uint32_t n, float* __restrict__ sel) {
     __shared__ uint32_t hist[256];
-    __shared__ uint32_t digit_s, rank_s;
     const float* a = arrays + (size_t)blockIdx.y * n;
-    uint32_t k = (n & 1u) ? n / 2 : n / 2 - 1 + blockIdx.x;
-    uint32_t prefix = 0, mask = 0;
-    for (int shift = 24; shift >= 0; shift -= 8) {
-        for (uint32_t i = threadIdx.x; i < 256; i += kSelBlock) hist[i] = 0;
-        __syncthreads();
-        for (uint32_t i = threadIdx.x; i < n; i += kSelBlock) {
-            const uint32_t u = __float_as_uint(__ldg(a + i));
-            if ((u & mask) == prefix) atomicAdd(&hist[(u >> shift) & 255u], 1u);
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            uint32_t below = 0, d = 0;
-            for (; d < 255; ++d) {
-                if (below + hist[d] > k) break;
-                below += hist[d];
-            }
-            digit_s = d;
-            rank_s = k - below;
-        }
-        __syncthreads();
-        prefix |= digit_s << shift;
-        mask |= 0xffu << shift;
-        k = rank_s;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) sel[blockIdx.y * 2 + blockIdx.x] = __uint_as_float(prefix);
+    const uint32_t k = (n & 1u) ? n / 2 : n / 2 - 1 + blockIdx.x;
+    uint32_t ties;
+    const uint32_t v = radix_select<kSelBlock>([a](uint32_t i) { return __float_as_uint(__ldg(a + i)); }, n, k,
+                                               hist, ties);
+    if (threadIdx.x == 0) sel[blockIdx.y * 2 + blockIdx.x] = __uint_as_float(v);
 }
 
 __device__ __forceinline__ float median_of(const float* sel, uint32_t n) {

@@ -15,6 +15,7 @@
 
 #include "common.cuh"
 #include "lidar_dir.cuh"
+#include "radix_select.cuh"
 
 namespace {
 
@@ -75,6 +76,86 @@ k_camera_rays(const float* __restrict__ pose, const int64_t* __restrict__ inds, 
     const float xs = __fdiv_rn(__fsub_rn(i, cx), fx), ys = __fdiv_rn(__fsub_rn(j, cy), fy);
     const float nrm = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(xs, xs), __fmul_rn(ys, ys)), 1.0f));
     emit_ray(P, __fdiv_rn(xs, nrm), __fdiv_rn(ys, nrm), __fdiv_rn(1.0f, nrm), k, rays_o, rays_d);
+}
+
+// ------------------------------------------------------------------------------- error-map sampling
+// torch-ngp's error-map branch of get_rays: N distinct coarse cells of a res x res map drawn with
+// probability proportional to the map (torch.multinomial without replacement), then one jittered pixel
+// inside each cell.  Exponential race: the N smallest keys E_i / w_i are such a draw.  Cells with
+// w <= 0 or non-finite w get the key E_i with the sign bit set, so as unsigned integers they order after
+// every positive-weight key: the N smallest keys are then the positive cells' draw, filled when there are
+// fewer than N positive cells by the smallest E among the rest.  One CTA per map holds the R = res^2 keys
+// in shared memory, radix-selects the N-th smallest and compacts the selected cells in ascending cell
+// order (ties at the N-th key go to the lower cells).
+constexpr int kEmBlock = 1024;
+
+// Exclusive count of `flag` over the CTA in thread order; *total = the CTA's count.  `warp_off` holds
+// kEmBlock / 32 + 1 words of shared memory.
+__device__ __forceinline__ uint32_t block_exclusive_count(bool flag, uint32_t* warp_off, uint32_t& total) {
+    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const uint32_t bal = __ballot_sync(0xffffffffu, flag);
+    __syncthreads();  // `warp_off` may still be read from the previous call
+    if (lane == 0) warp_off[warp] = __popc(bal);
+    __syncthreads();
+    if (tid < 32) {
+        const uint32_t c = warp_off[tid];
+        const uint32_t inc = warp_inclusive_scan(c, lane);
+        warp_off[tid] = inc - c;
+        if (tid == 31) warp_off[kEmBlock / 32] = inc;
+    }
+    __syncthreads();
+    total = warp_off[kEmBlock / 32];
+    return warp_off[warp] + __popc(bal & ((1u << lane) - 1u));
+}
+
+__global__ void __launch_bounds__(kEmBlock)
+k_error_map_sample(const float* __restrict__ error_map, const float* __restrict__ expo,
+                   const float* __restrict__ jitter, uint32_t res, uint32_t N, uint32_t H, uint32_t W,
+                   int64_t* __restrict__ inds_coarse, int64_t* __restrict__ inds) {
+    extern __shared__ uint32_t keys[];
+    __shared__ uint32_t hist[256];
+    __shared__ uint32_t warp_off[kEmBlock / 32 + 1];
+    const uint32_t R = res * res, tid = threadIdx.x;
+    for (uint32_t i = tid; i < R; i += kEmBlock) {
+        const float w = __ldg(error_map + i), e = __ldg(expo + i);
+        keys[i] = w > 0.f && w < INFINITY ? __float_as_uint(__fdiv_rn(e, w)) : 0x80000000u | __float_as_uint(e);
+    }
+    __syncthreads();
+    uint32_t ties;
+    const uint32_t T = radix_select<kEmBlock>([](uint32_t i) { return keys[i]; }, R, N - 1, hist, ties);
+    // torch-ngp: row = (cr * sx + u0 * sx).long().clamp(max=H-1), sx = H / res in fp32; cols with W
+    const float sx = (float)((double)H / (double)res), sy = (float)((double)W / (double)res);
+    uint32_t tie_base = 0, out_base = 0;
+    for (uint32_t c0 = 0; c0 < R && out_base < N; c0 += kEmBlock) {
+        const uint32_t i = c0 + tid;
+        const uint32_t u = i < R ? keys[i] : 0u;
+        const bool tie = i < R && u == T;
+        uint32_t n_tie, n_take;
+        const uint32_t tie_rank = tie_base + block_exclusive_count(tie, warp_off, n_tie);
+        const bool take = i < R && (u < T || (tie && tie_rank <= ties));
+        const uint32_t j = out_base + block_exclusive_count(take, warp_off, n_take);
+        if (take) {
+            const float u0 = __ldg(jitter + 2 * (size_t)j), u1 = __ldg(jitter + 2 * (size_t)j + 1);
+            const float r = __fadd_rn(__fmul_rn((float)(i / res), sx), __fmul_rn(u0, sx));
+            const float c = __fadd_rn(__fmul_rn((float)(i % res), sy), __fmul_rn(u1, sy));
+            const int64_t row = min((int64_t)r, (int64_t)H - 1), col = min((int64_t)c, (int64_t)W - 1);
+            inds_coarse[j] = (int64_t)i;
+            inds[j] = row * W + col;
+        }
+        tie_base += n_tie;
+        out_base += n_take;
+    }
+}
+
+// torch-ngp train_step: map[c_j] = 0.1 * map[c_j] + 0.9 * loss[j] over one batch row's distinct cells.
+__global__ void __launch_bounds__(256)
+k_error_map_update(float* __restrict__ error_map, uint32_t R, const int64_t* __restrict__ inds_coarse,
+                   uint32_t N, const float* __restrict__ loss) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= N) return;
+    const int64_t c = __ldg(inds_coarse + j);
+    if (c < 0 || c >= (int64_t)R) return;  // never write outside the map
+    error_map[c] = __fadd_rn(__fmul_rn(0.1f, error_map[c]), __fmul_rn(0.9f, __ldg(loss + j)));
 }
 
 // ---------------------------------------------------------------------------------- occupancy grid
@@ -243,6 +324,28 @@ int nvsf_get_rays(const float* pose, const int64_t* inds, uint32_t n, uint32_t H
         return NVSF_E_INVALID;
     k_camera_rays<<<nvsf_div_up(n, 256u), 256, 0, (cudaStream_t)stream>>>(
         pose, inds, n, H, W, fx, fy, cx, cy, rays_o, rays_d);
+    return nvsf_launch_status();
+}
+
+int nvsf_error_map_sample(const float* error_map, const float* expo, const float* jitter, uint32_t res,
+                          uint32_t N, uint32_t H, uint32_t W, int64_t* inds_coarse, int64_t* inds, void* stream) {
+    if (!error_map || !expo || !jitter || !inds_coarse || !inds || res == 0 || res > NVSF_ERROR_MAP_MAX_RES ||
+        H == 0 || W == 0 || N == 0 || N > res * res)
+        return NVSF_E_INVALID;
+    const size_t smem = (size_t)res * res * sizeof(uint32_t);
+    const cudaError_t e =
+        cudaFuncSetAttribute(k_error_map_sample, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    k_error_map_sample<<<1, kEmBlock, smem, (cudaStream_t)stream>>>(error_map, expo, jitter, res, N, H, W,
+                                                                    inds_coarse, inds);
+    return nvsf_launch_status();
+}
+
+int nvsf_error_map_update(float* error_map, uint32_t R, const int64_t* inds_coarse, uint32_t N, const float* loss,
+                          void* stream) {
+    if (N == 0) return NVSF_OK;
+    if (!error_map || !inds_coarse || !loss || R == 0) return NVSF_E_INVALID;
+    k_error_map_update<<<nvsf_div_up(N, 256u), 256, 0, (cudaStream_t)stream>>>(error_map, R, inds_coarse, N, loss);
     return nvsf_launch_status();
 }
 
