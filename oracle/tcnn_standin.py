@@ -77,18 +77,21 @@ class _HashGrid(nn.Module):
         self.params = nn.Parameter(p)
 
     def forward(self, x):
-        x = x.to(torch.float32)
+        # float32 like tcnn; float64 inputs stay float64 (tests/test_encoder_bwd_oracle.py differentiates the
+        # encoders in float64) — the table is still the fp16-rounded parameters either way
+        dt = torch.float64 if x.dtype == torch.float64 else torch.float32
+        x = x.to(dt)
         N = x.shape[0]
-        table = _fp16_round(self.params).view(-1, self.F)
+        table = _fp16_round(self.params).to(dt).view(-1, self.F)
         outs = []
         for lv in self.levels:
             pos = x * np.float32(lv["scale"]) + 0.5
             cell = torch.floor(pos)
             w = pos - cell
             cell = cell.to(torch.int64)
-            acc = torch.zeros(N, self.F, dtype=torch.float32)
+            acc = torch.zeros(N, self.F, dtype=dt)
             for corner in range(1 << self.D):
-                weight = torch.ones(N, dtype=torch.float32)
+                weight = torch.ones(N, dtype=dt)
                 idx_dense = torch.zeros(N, dtype=torch.int64)
                 idx_hash = torch.zeros(N, dtype=torch.int64)
                 stride = 1

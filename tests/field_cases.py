@@ -72,8 +72,9 @@ def linear_loss(out, coef, to=lambda a: torch.from_numpy(a)):
             + (to(coef["c"]) * out["weights"]).sum() + (to(coef["e"]) * out["weights_sum"]).sum())
 
 
-def oracle_grads(case, params=None):
-    """Autograd gradients of the CPU oracle for one gradient case, in the flat parameter layout."""
+def oracle_grads(case, params=None, bg_color=1.0):
+    """Autograd gradients of the CPU oracle for one gradient case, in the flat parameter layout (camera:
+    background `bg_color`, a number or an [N,3] tensor)."""
     from oracle.field_oracle import FieldOracle
     from oracle import raymarching_oracle as RO
     base = params if params is not None else oracle_params()
@@ -88,7 +89,7 @@ def oracle_grads(case, params=None):
         nears, fars = torch.from_numpy(n), torch.from_numpy(f)
     S_ = case["coef"]["c"].shape[1]
     out = orc.run(torch.from_numpy(case["o"]), torch.from_numpy(case["d"]), case["t"], case["lidar"], S_, nears,
-                  fars, None if case["noise"] is None else torch.from_numpy(case["noise"]))
+                  fars, None if case["noise"] is None else torch.from_numpy(case["noise"]), bg_color=bg_color)
     loss = linear_loss(out, case["coef"])
     (loss * LOSS_SCALE).backward()   # the goldens were taken with this loss scale (oracle/make_golden_grad.py)
     un = lambda v: (v.grad / LOSS_SCALE if v.grad is not None else torch.zeros_like(v)).numpy()
