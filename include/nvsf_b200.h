@@ -33,7 +33,7 @@ extern "C" {
 #define NVSF_E_WORKSPACE (-2) /* workspace too small */
 
 /* ABI version of this header; bumped on any signature change. */
-#define NVSF_B200_ABI_VERSION 15
+#define NVSF_B200_ABI_VERSION 16
 int nvsf_abi_version(void);
 /* Human-readable text for a status returned by any nvsf_* call. */
 const char* nvsf_status_string(int status);
@@ -629,6 +629,30 @@ int nvsf_eval_lidar(const float* depth, const float* image, const float* gt, uin
 size_t nvsf_eval_camera_workspace_bytes(uint32_t H, uint32_t W);
 int nvsf_eval_camera(const float* pred, const float* gt, uint32_t H, uint32_t W, float* row, void* workspace,
                      size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------- */
+/* Part 7 — mesh extraction                                                   */
+/* ------------------------------------------------------------------------- */
+/* Replaces mcubes.marching_cubes in torch-ngp's save_mesh (the reference's UtilsTrainer).  Contract: DESIGN.md
+ * §3.5.  volume [X,Y,Z] fp32 C-contiguous, u[i,j,k] = lattice point (i,j,k), each of X, Y, Z in [2, 1024].  A
+ * point is above when u > threshold (NaN is not above).
+ *   vertices [V,3] fp32, in index space: one per lattice edge (a, b) whose endpoints differ in "above", ordered by
+ *     the owning point's linear index (i*Y + j)*Z + k (a point owns its +x, +y, +z edges) and then by axis; the
+ *     edge's axis coordinate is float(index) + t, t = clamp((threshold - u_a) / (u_b - u_a), 0, 1) in IEEE fp32
+ *     (fminf(fmaxf(t, 0), 1): a non-finite t lands on a).  Shared between cells, no duplicates.
+ *   triangles [T,3] int64 into vertices: per cell (i < X-1, j < Y-1, k < Z-1) in linear order, the cell's case
+ *     (csrc/mc_tables.cuh, generated by oracle/make_mc_tables.py) in table order; the normal
+ *     (v1 - v0) x (v2 - v0) points out of the above region.  The surface is closed away from the volume boundary.
+ * Two phases: _count writes counts[0] = V, counts[1] = T (device int64); after it, _write with the same volume,
+ * threshold and workspace writes the rows below v_cap / t_cap (a NULL output is allowed with a zero cap).  No
+ * atomics and no float reductions: the output is bit-identical from run to run.
+ * workspace (16-byte aligned): 4 bytes per lattice point plus 8 per 1024 points (4.0 GiB at 1024^3). */
+size_t nvsf_marching_cubes_workspace_bytes(uint32_t X, uint32_t Y, uint32_t Z);
+int nvsf_marching_cubes_count(const float* volume, uint32_t X, uint32_t Y, uint32_t Z, float threshold,
+                              int64_t* counts, void* workspace, size_t workspace_bytes, void* stream);
+int nvsf_marching_cubes_write(const float* volume, uint32_t X, uint32_t Y, uint32_t Z, float threshold,
+                              float* vertices, uint64_t v_cap, int64_t* triangles, uint64_t t_cap, void* workspace,
+                              size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -14,6 +14,7 @@ Sub-modules
     losses        lidar_loss / rgb_loss of the reference's train_step, loss + derivative in one kernel
     chamfer       drop-in for reference ``nvsf.nerf.chamfer3D.dist_chamfer_3D`` (chamfer_3DDist)
     metrics       evaluation on the device: lidar_points (range image -> point cloud), LidarMeter / CameraMeter
+    mesh          mesh extraction: marching_cubes on the device (drop-in for mcubes) and write_ply
     _lib          ctypes binding of the C ABI (include/nvsf_b200.h)
     build         compiles csrc/*.cu into libnvsf_b200.so with nvcc (sm_100a)
 """
@@ -26,6 +27,7 @@ from . import optim  # noqa: F401
 from . import losses  # noqa: F401
 from . import chamfer  # noqa: F401
 from . import metrics  # noqa: F401
+from . import mesh  # noqa: F401
 from .field import NeRFNetwork  # noqa: F401
 
 __version__ = "0.1.0"

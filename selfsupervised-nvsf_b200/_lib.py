@@ -122,6 +122,11 @@ PROTOTYPES = {
     "nvsf_eval_lidar": (_int, [_p, _p, _p, _u32, _u32, _f32, _f32, _f32, _f32, _f32, _f32, _p, _p, _sz, _p]),
     "nvsf_eval_camera_workspace_bytes": (_sz, [_u32, _u32]),
     "nvsf_eval_camera": (_int, [_p, _p, _u32, _u32, _p, _p, _sz, _p]),
+    # Part 7 — mesh extraction
+    "nvsf_marching_cubes_workspace_bytes": (_sz, [_u32, _u32, _u32]),
+    "nvsf_marching_cubes_count": (_int, [_p, _u32, _u32, _u32, _f32, _p, _p, _sz, _p]),
+    "nvsf_marching_cubes_write": (_int, [_p, _u32, _u32, _u32, _f32, _p, ctypes.c_uint64, _p, ctypes.c_uint64, _p,
+                                         _sz, _p]),
 }
 
 _lib = None
@@ -154,7 +159,7 @@ def lib():
     return _lib
 
 
-ABI_VERSION = 15
+ABI_VERSION = 16
 
 
 def check(status, what=""):

@@ -28,6 +28,15 @@ __device__ __forceinline__ uint32_t warp_inclusive_scan(uint32_t v, int lane) {
     return v;
 }
 
+__device__ __forceinline__ uint64_t warp_inclusive_scan(uint64_t v, int lane) {
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        uint64_t o = __shfl_up_sync(0xffffffffu, v, d);
+        if (lane >= d) v += o;
+    }
+    return v;
+}
+
 __device__ __forceinline__ uint32_t warp_reduce_sum(uint32_t v) {
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);

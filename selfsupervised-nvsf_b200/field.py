@@ -780,6 +780,41 @@ class NeRFNetwork(nn.Module):
         st["iter_density"] += 1
         return st["density_bitfield"]
 
+    @torch.no_grad()
+    @_lib.device_guard
+    @_lib.with_options
+    def extract_geometry(self, time, resolution=256, threshold=10.0, cal_lidar_color=False):
+        """torch-ngp's extract_geometry / save_mesh on the device: sigma at `time` on the resolution^3 lattice
+        torch.linspace(aabb_infer[a], aabb_infer[3 + a], resolution) per axis ('ij' order), marching cubes at
+        `threshold` (mesh.marching_cubes) and the vertex transform v / (resolution - 1) * (b_max - b_min) + b_min
+        in fp32.  Returns (vertices [V,3] fp32 world coordinates, triangles [T,3] int64), both on the device."""
+        from . import mesh
+        R = int(resolution)
+        vol, b = self._density_volume(time, R, bool(cal_lidar_color))
+        v, f = mesh.marching_cubes(vol, threshold)
+        lo, hi = b[:3].to(vol.device), b[3:].to(vol.device)
+        return v / float(R - 1) * (hi - lo) + lo, f
+
+    @torch.no_grad()
+    @_lib.device_guard
+    @_lib.with_options
+    def _density_volume(self, time, R, lidar):
+        """(sigma [R,R,R] on the device, aabb_infer on the host): x-slabs of at most 2^24 lattice points."""
+        if not 2 <= R <= 1024:
+            raise _lib.NvsfError(f"extract_geometry: resolution {R} out of range [2, 1024]")
+        dev = self.sigma_net.device
+        b = self.aabb_infer.detach().to(torch.float32).cpu()
+        axes = [torch.linspace(b[a], b[3 + a], R).to(dev) for a in range(3)]   # the reference's CPU linspace
+        vol = torch.empty(R, R, R, dtype=torch.float32, device=dev)
+        self.prepare(time, lidar)
+        slab = max(1, (1 << 24) // (R * R))
+        for i0 in range(0, R, slab):
+            xs = axes[0][i0:i0 + slab]
+            pts = torch.stack(torch.meshgrid(xs, axes[1], axes[2], indexing="ij"), -1).view(-1, 3)
+            sigma, _, _, _ = self._density_raw(pts, time, lidar, prepared=True)
+            vol[i0:i0 + len(xs)].view(-1).copy_(sigma)
+        return vol, b
+
     # ------------------------------------------------------------------ march_rays* render loops
     @torch.no_grad()
     @_lib.device_guard
