@@ -33,7 +33,7 @@ extern "C" {
 #define NVSF_E_WORKSPACE (-2) /* workspace too small */
 
 /* ABI version of this header; bumped on any signature change. */
-#define NVSF_B200_ABI_VERSION 16
+#define NVSF_B200_ABI_VERSION 17
 int nvsf_abi_version(void);
 /* Human-readable text for a status returned by any nvsf_* call. */
 const char* nvsf_status_string(int status);
@@ -598,6 +598,23 @@ size_t nvsf_lidar_points_workspace_bytes(uint32_t H, uint32_t W);
 int nvsf_lidar_points(const float* depth, const float* raydrop, float raydrop_threshold, const float* intensity,
                       uint32_t H, uint32_t W, float fov_up, float fov, float fov_hoz, float scale, float* points,
                       int32_t* count, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Point cloud -> range image (the inverse of nvsf_lidar_points; the images_lidar ground truth).  Scan b is rows
+ * [offsets[b], offsets[b+1]) of points [P, channels] (x, y, z[, intensity], fp32; offsets device int64 [B+1],
+ * non-decreasing, every scan < 2^32 points and <= max_count).  With poses [B,16] (lidar2world, row-major, rigid;
+ * NULL = points already in the sensor frame) a point is first taken to R^T (p - t).  In float64, each operation
+ * rounded on its own: depth32 = fp32(|q|), kept when 0 < depth32 < max_depth (NaN / inf dropped);
+ * beta = atan2(q_y, q_x), alpha = atan2(q_z, |q_xy|) in degrees; c = rint((0.5 fov_hoz - beta) / fov_hoz * W),
+ * r = rint((fov_up - alpha) / fov * H) (half to even), kept when inside the frame (the seam half-column at c = W is
+ * dropped, not wrapped).  Per pixel the smallest depth32 wins, ties to the lowest index in the scan.
+ * images [B,H,W,3]: (1, intensity or 0, depth32 * scale) at a hit, (0, 0, 0) elsewhere; index [B,H,W] (may be
+ * NULL): the winner's row in points, or -1.  Bit-identical from run to run.  H*W <= 2^26, B <= 65535.
+ * workspace (8-byte aligned): nvsf_range_image_workspace_bytes = 8 bytes per pixel of the batch. */
+size_t nvsf_range_image_workspace_bytes(uint32_t B, uint32_t H, uint32_t W);
+int nvsf_range_image(const float* points, uint32_t channels, const int64_t* offsets, uint32_t B, uint32_t max_count,
+                     const float* poses, uint32_t H, uint32_t W, float fov_up, float fov, float fov_hoz, float scale,
+                     float max_depth, float* images, int64_t* index, void* workspace, size_t workspace_bytes,
+                     void* stream);
 
 /* One LiDAR frame's metric row (NVSF_EVAL_LIDAR_K floats, column order below).  depth [H,W] and image [H,W,2]
  * (raydrop probability, intensity) are render_frame's outputs; gt [H,W,3] = (raydrop mask, intensity, depth)

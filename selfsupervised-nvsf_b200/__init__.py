@@ -13,7 +13,8 @@ Sub-modules
     optim         Adam over the flat parameter / gradient buffers (CUDA kernel)
     losses        lidar_loss / rgb_loss of the reference's train_step, loss + derivative in one kernel
     chamfer       drop-in for reference ``nvsf.nerf.chamfer3D.dist_chamfer_3D`` (chamfer_3DDist)
-    metrics       evaluation on the device: lidar_points (range image -> point cloud), LidarMeter / CameraMeter
+    metrics       evaluation on the device: lidar_points (range image -> point cloud), range_image (point cloud ->
+                  range image, the images_lidar ground truth), LidarMeter / CameraMeter
     mesh          mesh extraction: marching_cubes on the device (drop-in for mcubes) and write_ply
     _lib          ctypes binding of the C ABI (include/nvsf_b200.h)
     build         compiles csrc/*.cu into libnvsf_b200.so with nvcc (sm_100a)

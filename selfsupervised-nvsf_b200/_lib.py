@@ -118,6 +118,9 @@ PROTOTYPES = {
     "nvsf_chamfer_forward_counted": (_int, [_p, _p, _u32, _u32, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "nvsf_lidar_points_workspace_bytes": (_sz, [_u32, _u32]),
     "nvsf_lidar_points": (_int, [_p, _p, _f32, _p, _u32, _u32, _f32, _f32, _f32, _f32, _p, _p, _p, _sz, _p]),
+    "nvsf_range_image_workspace_bytes": (_sz, [_u32, _u32, _u32]),
+    "nvsf_range_image": (_int, [_p, _u32, _p, _u32, _u32, _p, _u32, _u32, _f32, _f32, _f32, _f32, _f32, _p, _p, _p,
+                                _sz, _p]),
     "nvsf_eval_lidar_workspace_bytes": (_sz, [_u32, _u32]),
     "nvsf_eval_lidar": (_int, [_p, _p, _p, _u32, _u32, _f32, _f32, _f32, _f32, _f32, _f32, _p, _p, _sz, _p]),
     "nvsf_eval_camera_workspace_bytes": (_sz, [_u32, _u32]),
@@ -159,7 +162,7 @@ def lib():
     return _lib
 
 
-ABI_VERSION = 16
+ABI_VERSION = 17
 
 
 def check(status, what=""):

@@ -121,6 +121,106 @@ void launch_points(const float* depth, const float* raydrop, float thr, const fl
                                                counts, points, count);
 }
 
+// --------------------------------------------------------------------------------- point cloud -> range image
+// The nearest return of each pixel, ties to the lowest point index: one 64-bit key per pixel, (depth32 bits << 32 |
+// index within the scan), lowered by atomicMin (depth32 > 0, so its fp32 bits order as integers); 0xFF..FF = empty.
+// Float64 arithmetic in the contract's order (DESIGN.md §3.5), every operation rounded on its own.
+constexpr int kRiBlock = 256;
+constexpr unsigned long long kRiEmpty = ~0ull;
+constexpr uint32_t kRiNoPixel = 0xFFFFFFFFu;  // above every pixel id (H*W <= 2^26)
+
+__device__ __forceinline__ double ri_col_or_row(double num, double den, uint32_t n) {
+    return rint(__dmul_rn(__ddiv_rn(num, den), (double)n));
+}
+
+// Grid (point blocks, scans), blockIdx.x fastest: the blocks in flight cover one or two scans, whose keys stay in L2.
+__global__ void __launch_bounds__(kRiBlock)
+k_range_scatter(const float* __restrict__ points, uint32_t channels, const int64_t* __restrict__ offsets,
+                const float* __restrict__ poses, uint32_t H, uint32_t W, float fov_up, float fov, float fov_hoz,
+                float max_depth, unsigned long long* __restrict__ keys) {
+    __shared__ double pose_s[12];  // rows 0..2 of lidar2world: R | t
+    const uint32_t b = blockIdx.y;
+    const int64_t begin = offsets[b], count = offsets[b + 1] - begin;
+    if ((int64_t)blockIdx.x * kRiBlock >= count) return;
+    if (poses && threadIdx.x < 12) pose_s[threadIdx.x] = (double)poses[(size_t)b * 16 + threadIdx.x];
+    __syncthreads();
+    const uint32_t i = blockIdx.x * kRiBlock + threadIdx.x;
+    uint32_t pix = kRiNoPixel;
+    float depth32 = 0.f;
+    if ((int64_t)i < count) {
+        const float* p = points + (size_t)(begin + i) * channels;
+        double qx = (double)__ldg(p), qy = (double)__ldg(p + 1), qz = (double)__ldg(p + 2);
+        if (poses) {  // R^T (p - t)
+            const double dx = __dsub_rn(qx, pose_s[3]), dy = __dsub_rn(qy, pose_s[7]), dz = __dsub_rn(qz, pose_s[11]);
+            qx = __dadd_rn(__dadd_rn(__dmul_rn(pose_s[0], dx), __dmul_rn(pose_s[4], dy)), __dmul_rn(pose_s[8], dz));
+            qy = __dadd_rn(__dadd_rn(__dmul_rn(pose_s[1], dx), __dmul_rn(pose_s[5], dy)), __dmul_rn(pose_s[9], dz));
+            qz = __dadd_rn(__dadd_rn(__dmul_rn(pose_s[2], dx), __dmul_rn(pose_s[6], dy)), __dmul_rn(pose_s[10], dz));
+        }
+        const double xy2 = __dadd_rn(__dmul_rn(qx, qx), __dmul_rn(qy, qy));
+        depth32 = __double2float_rn(__dsqrt_rn(__dadd_rn(xy2, __dmul_rn(qz, qz))));
+        if (depth32 > 0.f && depth32 < max_depth) {  // false for NaN; inf is never below max_depth
+            const double kDeg = 180.0 / 3.14159265358979323846;
+            const double beta = __dmul_rn(atan2(qy, qx), kDeg), alpha = __dmul_rn(atan2(qz, __dsqrt_rn(xy2)), kDeg);
+            const double fh = (double)fov_hoz;
+            const double c = ri_col_or_row(__dsub_rn(__dmul_rn(0.5, fh), beta), fh, W);
+            const double r = ri_col_or_row(__dsub_rn((double)fov_up, alpha), (double)fov, H);
+            // the seam half-column that rounds to c = W is dropped, as the reference loop drops it
+            if (c >= 0.0 && c < (double)W && r >= 0.0 && r < (double)H) pix = (uint32_t)r * W + (uint32_t)c;
+        }
+    }
+    const unsigned long long key = ((unsigned long long)__float_as_uint(depth32) << 32) | i;
+    // Same-address reductions serialise; lanes of a warp that share a pixel (an accumulated cloud, a point
+    // repeated, a scan in firing order) first take their minimum by pointer jumping along the lanes of their group,
+    // and the lowest lane issues the one reduction.  The grouping (MATCH.ANY) costs ~10 % on a scan of distinct
+    // pixels, so it only runs in a warp where two neighbouring lanes share a pixel.
+    const uint32_t lane = threadIdx.x & 31;
+    const uint32_t prev = __shfl_up_sync(0xffffffffu, pix, 1);
+    unsigned long long kmin = key;
+    bool lead = true;
+    if (__any_sync(0xffffffffu, lane > 0 && prev == pix && pix != kRiNoPixel)) {
+        const uint32_t peers = __match_any_sync(0xffffffffu, pix);
+        lead = (peers & ((1u << lane) - 1u)) == 0;
+        const uint32_t above = peers & ~((2u << lane) - 1u);
+        int next = above ? __ffs(above) - 1 : -1;
+#pragma unroll
+        for (int step = 0; step < 5; ++step) {
+            const int src = next >= 0 ? next : (int)lane;
+            const unsigned long long k2 = __shfl_sync(0xffffffffu, kmin, src);
+            const int n2 = __shfl_sync(0xffffffffu, next, src);
+            if (next >= 0) {
+                kmin = k2 < kmin ? k2 : kmin;
+                next = n2;
+            }
+        }
+    }
+    if (pix != kRiNoPixel && lead)
+        atomicMin(keys + (size_t)b * H * W + pix, kmin);  // result unused: a RED, not an ATOM
+}
+
+// One thread per pixel: the winner's row (1, intensity or 0, depth32 * scale) and its global point row, or
+// (0, 0, 0) and -1 for an empty pixel.
+__global__ void __launch_bounds__(kRiBlock)
+k_range_resolve(const unsigned long long* __restrict__ keys, const float* __restrict__ points, uint32_t channels,
+                const int64_t* __restrict__ offsets, uint32_t n, float scale, float* __restrict__ images,
+                int64_t* __restrict__ index) {
+    const uint32_t p = blockIdx.x * kRiBlock + threadIdx.x;
+    if (p >= n) return;
+    const size_t g = (size_t)blockIdx.y * n + p;
+    const unsigned long long k = keys[g];
+    float m = 0.f, it = 0.f, d = 0.f;
+    int64_t row = -1;
+    if (k != kRiEmpty) {
+        row = offsets[blockIdx.y] + (int64_t)(uint32_t)k;
+        m = 1.f;
+        if (channels == 4) it = __ldg(points + (size_t)row * 4 + 3);
+        d = __fmul_rn(__uint_as_float((uint32_t)(k >> 32)), scale);
+    }
+    images[3 * g] = m;
+    images[3 * g + 1] = it;
+    images[3 * g + 2] = d;
+    if (index) index[g] = row;
+}
+
 // ------------------------------------------------------------------------------------------ LiDAR pixel pass
 // Per pixel, with m^ = (raydrop^ > 0.5): P = D^ m^ / scale, G = D r / scale (unclamped: the point clouds),
 // clamped copies for depth [1e-3, max_depth] and intensity I^ = i^ m^, I = i r in [1e-6, 1] (the SSIM images),
@@ -446,6 +546,32 @@ int nvsf_lidar_points(const float* depth, const float* raydrop, float raydrop_th
     if (workspace_bytes < nvsf_lidar_points_workspace_bytes(H, W)) return NVSF_E_WORKSPACE;
     launch_points(depth, raydrop, raydrop_threshold, intensity, H, W, fov_up, fov, fov_hoz, scale, points, count,
                   reinterpret_cast<uint32_t*>(workspace), (cudaStream_t)stream);
+    return nvsf_launch_status();
+}
+
+size_t nvsf_range_image_workspace_bytes(uint32_t B, uint32_t H, uint32_t W) {
+    return frame_ok(H, W) ? (size_t)B * H * W * sizeof(unsigned long long) : 0;
+}
+
+int nvsf_range_image(const float* points, uint32_t channels, const int64_t* offsets, uint32_t B, uint32_t max_count,
+                     const float* poses, uint32_t H, uint32_t W, float fov_up, float fov, float fov_hoz, float scale,
+                     float max_depth, float* images, int64_t* index, void* workspace, size_t workspace_bytes,
+                     void* stream) {
+    if ((channels != 3 && channels != 4) || !frame_ok(H, W) || B > 65535u) return NVSF_E_INVALID;
+    if (B == 0) return NVSF_OK;
+    if (!offsets || !images || !workspace || (max_count && !points)) return NVSF_E_INVALID;
+    if (reinterpret_cast<uintptr_t>(workspace) & 7u) return NVSF_E_INVALID;
+    if (workspace_bytes < nvsf_range_image_workspace_bytes(B, H, W)) return NVSF_E_WORKSPACE;
+    cudaStream_t s = (cudaStream_t)stream;
+    auto* keys = reinterpret_cast<unsigned long long*>(workspace);
+    const uint32_t n = H * W;
+    cudaError_t e = cudaMemsetAsync(keys, 0xFF, (size_t)B * n * sizeof(unsigned long long), s);
+    if (e != cudaSuccess) return (int)e;
+    if (max_count)
+        k_range_scatter<<<dim3((uint32_t)nvsf_div_up<uint64_t>(max_count, kRiBlock), B), kRiBlock, 0, s>>>(
+            points, channels, offsets, poses, H, W, fov_up, fov, fov_hoz, max_depth, keys);
+    k_range_resolve<<<dim3(nvsf_div_up(n, (uint32_t)kRiBlock), B), kRiBlock, 0, s>>>(keys, points, channels, offsets, n,
+                                                                                      scale, images, index);
     return nvsf_launch_status();
 }
 

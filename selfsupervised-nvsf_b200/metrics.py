@@ -1,6 +1,7 @@
-"""Evaluation of rendered frames on the device: the synthesized LiDAR scan (range image -> point cloud) and
-the per-frame meters of the reference's evaluation (Trainer.evaluate_one_epoch / test_step, trainer.py:817-903,
-1458-1846, meters nvsf/lib/error_matrices.py, conversion nvsf/lib/convert.py), over C ABI Part 6 (csrc/eval.cu).
+"""Evaluation of rendered frames on the device: the synthesized LiDAR scan (range image -> point cloud), its
+inverse (point cloud -> range image: the images_lidar ground truth) and the per-frame meters of the reference's
+evaluation (Trainer.evaluate_one_epoch / test_step, trainer.py:817-903, 1458-1846, meters
+nvsf/lib/error_matrices.py, conversion nvsf/lib/convert.py), over C ABI Part 6 (csrc/eval.cu).
 
 The reference copies every rendered frame to the host and scores it with numpy; here a frame's scoring is a
 fixed sequence of kernels in the current stream that writes one metric row to device memory, so evaluation
@@ -61,6 +62,81 @@ def lidar_points(depth, intrinsics, intrinsics_hoz, scale=1.0, raydrop=None, int
     check(L.nvsf_lidar_points(ptr(d), ptr(r), float(raydrop_threshold), ptr(it), H, W, *_fovs(intrinsics, intrinsics_hoz),
                               float(scale), ptr(points), ptr(count), ptr(ws), wb, stream_ptr()), "lidar_points")
     return points, count
+
+
+def _scan_offsets(offsets, P):
+    """Host list of the scan boundaries [B+1]: 0, non-decreasing, P at the end, every scan < 2^32 points."""
+    if offsets is None:
+        return [0, P]
+    if torch.is_tensor(offsets):
+        if offsets.is_cuda:
+            raise NvsfError("range_image: offsets must be host ints (a list or a CPU tensor)")
+        offsets = offsets.tolist()
+    try:
+        offs = [int(o) for o in offsets]
+    except (TypeError, ValueError):
+        raise NvsfError("range_image: offsets must be a sequence of ints") from None
+    if len(offs) < 2 or offs[0] != 0 or offs[-1] != P:
+        raise NvsfError(f"range_image: offsets must start at 0 and end at {P} (the number of points)")
+    if any(b < a for a, b in zip(offs, offs[1:])):
+        raise NvsfError("range_image: offsets must be non-decreasing")
+    if any(b - a >= 1 << 32 for a, b in zip(offs, offs[1:])):
+        raise NvsfError("range_image: a scan has 2^32 points or more")
+    return offs
+
+
+@torch.no_grad()
+@_lib.device_guard
+def range_image(points, H, W, intrinsics, intrinsics_hoz, scale=1.0, max_depth=80.0, offsets=None, poses=None,
+                return_index=False):
+    """Point cloud -> range image, the images_lidar ground truth that lidar_loss and LidarMeter read (convert.py's
+    point-to-pano projection; the exact inverse of get_lidar_rays's pixel directions; contract DESIGN.md §3.5).
+
+    points [P, 3|4] CUDA fp32 (x, y, z[, intensity]).  offsets: host ints [B+1] (list or CPU tensor), scan b =
+    rows offsets[b]:offsets[b+1]; None = one scan.  poses: lidar2world [B,4,4] (or [4,4] for one scan) on the
+    device, or None for points in the sensor frame.  Per pixel the nearest point with 0 < depth < max_depth wins
+    (ties to the lowest index); images [B,H,W,3] (or [H,W,3] without offsets) = (1, intensity or 0, depth * scale)
+    at a hit and zeros elsewhere.  With return_index=True also index [B,H,W] (or [H,W]) int64, the winner's row in
+    `points` or -1.  Reads nothing back to the host."""
+    if not torch.is_tensor(points) or not points.is_cuda:
+        raise NvsfError("range_image: points must be a CUDA tensor")
+    if points.dtype != torch.float32 or points.dim() != 2 or points.shape[1] not in (3, 4):
+        raise NvsfError(f"range_image: points must be fp32 [P, 3|4], got {points.dtype} {tuple(points.shape)}")
+    H, W = int(H), int(W)
+    P, C = int(points.shape[0]), int(points.shape[1])
+    offs = _scan_offsets(offsets, P)
+    B = len(offs) - 1
+    if B > 65535:
+        raise NvsfError(f"range_image: {B} scans in one call (at most 65535)")
+    L = _lib.lib()
+    wb = L.nvsf_range_image_workspace_bytes(B, H, W) if H > 0 and W > 0 else 0
+    if wb == 0 and B > 0:
+        raise NvsfError(f"range_image: frame {H}x{W} out of range")
+    dev = points.device
+    pose_t = None
+    if poses is not None:
+        if not torch.is_tensor(poses) or not poses.is_cuda:
+            raise NvsfError("range_image: poses must be a CUDA tensor")
+        if poses.device != dev:
+            raise NvsfError(f"range_image: poses must be on {dev}")
+        if tuple(poses.shape) == (4, 4):
+            poses = poses[None]
+        if tuple(poses.shape) != (B, 4, 4):
+            raise NvsfError(f"range_image: poses {tuple(poses.shape)} do not match {B} scans ([B, 4, 4])")
+        pose_t = poses.to(torch.float32).contiguous()
+    pts = points.contiguous()
+    off_t = torch.tensor(offs, dtype=torch.int64).to(dev)
+    images = torch.empty(B, H, W, 3, dtype=torch.float32, device=dev)
+    index = torch.empty(B, H, W, dtype=torch.int64, device=dev) if return_index else None
+    ws = torch.empty(wb, dtype=torch.uint8, device=dev)
+    max_count = max((b - a for a, b in zip(offs, offs[1:])), default=0)
+    check(L.nvsf_range_image(ptr(pts), C, ptr(off_t), B, max_count, ptr(pose_t), H, W,
+                             *_fovs(intrinsics, intrinsics_hoz), float(scale), float(max_depth), ptr(images),
+                             ptr(index), ptr(ws), wb, stream_ptr()), "range_image")
+    if offsets is None:
+        images = images[0]
+        index = None if index is None else index[0]
+    return (images, index) if return_index else images
 
 
 def summarize(rows, names, process_group=None):
