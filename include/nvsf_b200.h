@@ -33,7 +33,7 @@ extern "C" {
 #define NVSF_E_WORKSPACE (-2) /* workspace too small */
 
 /* ABI version of this header; bumped on any signature change. */
-#define NVSF_B200_ABI_VERSION 17
+#define NVSF_B200_ABI_VERSION 18
 int nvsf_abi_version(void);
 /* Human-readable text for a status returned by any nvsf_* call. */
 const char* nvsf_status_string(int status);
@@ -260,6 +260,7 @@ int nvsf_field_color(const nvsf_field_config_t* cfg, const void* workspace, uint
  * memory, 0 = mma.sync; "enc_bwd_h16" (default 1) = product-rule texels from the fp16 plane mirrors;
  * "enc_bwd_ctas" (2 | 3); "bwd_shift_flow" / "_sigma" / "_heads" = extra binades of the fp16 gradient scale.
  * "march_mode", "composite_mode", "composite_bwd_mode" pick the operator kernel variants (default: per size).
+ * "chamfer_grid" picks the Chamfer forward's path (see nvsf_chamfer_forward; result-neutral).
  * In the C ABI these are process-wide switches that the launch code reads on the host at launch time (the
  * defaults are the fastest measured configuration).  The host mirror gives them per-model meaning: a
  * NeRFNetwork carries its own `options` and every one of its entry points (autograd backward included) runs
@@ -562,7 +563,13 @@ int nvsf_loss_patch(const float* pred_depth, const float* gt_depth, const float*
  * (:246-265).  xyz1 [b,n,3], xyz2 [b,m,3]; dist1 [b,n] / idx1 [b,n] = squared distance to and index
  * of the nearest point of xyz2 (first minimum, bit-identical to the reference kernel), dist2 / idx2
  * the other direction.  Backward ACCUMULATES into grad_xyz1 / grad_xyz2 (the reference wrapper
- * zero-fills them, dist_chamfer_3D.py:76-80); either may be NULL. */
+ * zero-fills them, dist_chamfer_3D.py:76-80); either may be NULL.
+ * Two paths with bit-identical results: the brute-force scan over every pair, and a uniform grid over each
+ * cloud (built on the device, no host read) searched ring by ring with a conservative stopping bound
+ * (DESIGN.md §3.5).  The forward picks the grid when n * m per batch element (capacities in the counted form)
+ * reaches 2^28 and the workspace is 16-byte aligned; option "chamfer_grid" overrides the choice (-1 automatic,
+ * the default; 0 never; 1 always).  A target cloud whose points crowd a few cells is scanned by brute force
+ * inside the grid path.  The workspace (nvsf_chamfer_workspace_bytes) covers either path. */
 size_t nvsf_chamfer_workspace_bytes(uint32_t b, uint32_t n, uint32_t m);
 int nvsf_chamfer_forward(const float* xyz1, const float* xyz2, uint32_t b, uint32_t n, uint32_t m,
                          float* dist1, float* dist2, int32_t* idx1, int32_t* idx2, void* workspace,
@@ -644,6 +651,18 @@ int nvsf_eval_lidar(const float* depth, const float* image, const float* gt, uin
  * the per-channel SSIMs with data range 1.  workspace (16-byte aligned): nvsf_eval_camera_workspace_bytes. */
 #define NVSF_EVAL_CAMERA_K 2
 size_t nvsf_eval_camera_workspace_bytes(uint32_t H, uint32_t W);
+
+/* The point metrics of LidarMeter for arbitrary clouds: pred [cap_p,3] and gt [cap_g,3] hold *n_pred / *n_gt
+ * (device int32, clamped to [0, capacity]) points followed by padding.  row[4] = (chamfer, fscore, points_pred,
+ * points_gt) with the definitions of nvsf_eval_lidar's columns NVSF_EVAL_CHAMFER.. NVSF_EVAL_POINTS_GT: mean
+ * squared nearest-neighbour distance both ways, F-score of the shares of squared distances below
+ * fscore_threshold, +inf / 0 when a cloud is empty.  workspace (16-byte aligned):
+ * nvsf_eval_points_workspace_bytes(cap_p, cap_g) (0 for a zero capacity or one above INT32_MAX). */
+#define NVSF_EVAL_POINTS_K 4
+size_t nvsf_eval_points_workspace_bytes(uint32_t cap_p, uint32_t cap_g);
+int nvsf_eval_points(const float* pred, uint32_t cap_p, const int32_t* n_pred, const float* gt, uint32_t cap_g,
+                     const int32_t* n_gt, float fscore_threshold, float* row, void* workspace, size_t workspace_bytes,
+                     void* stream);
 int nvsf_eval_camera(const float* pred, const float* gt, uint32_t H, uint32_t W, float* row, void* workspace,
                      size_t workspace_bytes, void* stream);
 

@@ -123,6 +123,8 @@ PROTOTYPES = {
                                 _sz, _p]),
     "nvsf_eval_lidar_workspace_bytes": (_sz, [_u32, _u32]),
     "nvsf_eval_lidar": (_int, [_p, _p, _p, _u32, _u32, _f32, _f32, _f32, _f32, _f32, _f32, _p, _p, _sz, _p]),
+    "nvsf_eval_points_workspace_bytes": (_sz, [_u32, _u32]),
+    "nvsf_eval_points": (_int, [_p, _u32, _p, _p, _u32, _p, _f32, _p, _p, _sz, _p]),
     "nvsf_eval_camera_workspace_bytes": (_sz, [_u32, _u32]),
     "nvsf_eval_camera": (_int, [_p, _p, _u32, _u32, _p, _p, _sz, _p]),
     # Part 7 — mesh extraction
@@ -162,7 +164,7 @@ def lib():
     return _lib
 
 
-ABI_VERSION = 17
+ABI_VERSION = 18
 
 
 def check(status, what=""):

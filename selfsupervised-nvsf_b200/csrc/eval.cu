@@ -407,15 +407,11 @@ __device__ __forceinline__ double ssim_mean(const double* partial, const SsimGri
 
 __device__ __forceinline__ double f1_of(double p, double r) { return p + r > 0.0 ? 2.0 * p * r / (p + r) : 0.0; }
 
-__global__ void __launch_bounds__(kFinBlock)
-k_lidar_finalize(const double* __restrict__ stats, const double* __restrict__ ssim_part, SsimGrid sg,
-                 const float* __restrict__ sel, uint32_t n, float max_depth, float fscore_threshold,
-                 const float* __restrict__ dist1, const float* __restrict__ dist2, const int32_t* __restrict__ counts,
-                 float* __restrict__ row) {
-    __shared__ double red[kFinBlock / 32];
-    const double ssim_d = ssim_mean(ssim_part, sg, 0, red);
-    const double ssim_i = ssim_mean(ssim_part, sg, 1, red);
-    const uint32_t np_ = (uint32_t)max(counts[0], 0), ng = (uint32_t)max(counts[1], 0);
+// The point metrics of both meters, from the squared nearest-neighbour distances of the np_ predicted and ng
+// ground-truth points: chamfer = mean dist1 + mean dist2, fscore = F1 of the shares below the threshold; +inf / 0
+// when a cloud is empty.  Called by the whole CTA; the results are valid in thread 0.
+__device__ void points_metrics(const float* __restrict__ dist1, const float* __restrict__ dist2, uint32_t np_,
+                               uint32_t ng, float fscore_threshold, double* red, double& chamfer, double& fscore) {
     double s1 = 0.0, s2 = 0.0, c1 = 0.0, c2 = 0.0;
     if (np_ && ng) {
         for (uint32_t i = threadIdx.x; i < np_; i += kFinBlock) {
@@ -431,22 +427,52 @@ k_lidar_finalize(const double* __restrict__ stats, const double* __restrict__ ss
     s2 = block_reduce<Op::Sum>(s2, red);
     c1 = block_reduce<Op::Sum>(c1, red);
     c2 = block_reduce<Op::Sum>(c2, red);
+    chamfer = INFINITY;
+    fscore = 0.0;
+    if (np_ && ng) {
+        chamfer = s1 / (double)np_ + s2 / (double)ng;
+        fscore = f1_of(c1 / (double)np_, c2 / (double)ng);
+    }
+}
+
+__global__ void __launch_bounds__(kFinBlock)
+k_lidar_finalize(const double* __restrict__ stats, const double* __restrict__ ssim_part, SsimGrid sg,
+                 const float* __restrict__ sel, uint32_t n, float max_depth, float fscore_threshold,
+                 const float* __restrict__ dist1, const float* __restrict__ dist2, const int32_t* __restrict__ counts,
+                 float* __restrict__ row) {
+    __shared__ double red[kFinBlock / 32];
+    const double ssim_d = ssim_mean(ssim_part, sg, 0, red);
+    const double ssim_i = ssim_mean(ssim_part, sg, 1, red);
+    const uint32_t np_ = (uint32_t)max(counts[0], 0), ng = (uint32_t)max(counts[1], 0);
+    double chamfer, fscore;
+    points_metrics(dist1, dist2, np_, ng, fscore_threshold, red, chamfer, fscore);
     if (threadIdx.x != 0) return;
     const double N = (double)n, md = (double)max_depth;
     const double mse_d = stats[kSqDepth] / N, mse_i = stats[kSqInt] / N;
     const double tp = stats[kTp], fp = stats[kFp], fn = stats[kFn];
     const double prec = tp + fp > 0.0 ? tp / (tp + fp) : 0.0, rec = tp + fn > 0.0 ? tp / (tp + fn) : 0.0;
-    double chamfer = INFINITY, fscore = 0.0;
-    if (np_ && ng) {
-        chamfer = s1 / (double)np_ + s2 / (double)ng;
-        fscore = f1_of(c1 / (double)np_, c2 / (double)ng);
-    }
     const double out[NVSF_EVAL_LIDAR_K] = {
         sqrt(mse_d), (double)median_of(sel, n), 10.0 * log10(md * md / mse_d), ssim_d,
         sqrt(mse_i), (double)median_of(sel + 2, n), 10.0 * log10(1.0 / mse_i), ssim_i,
         sqrt(stats[kSqDrop] / N), stats[kAgree] / N, f1_of(prec, rec),
         chamfer, fscore, (double)np_, (double)ng};
     for (int k = 0; k < NVSF_EVAL_LIDAR_K; ++k) row[k] = (float)out[k];
+}
+
+// row = (chamfer, fscore, points_pred, points_gt) of two clouds with device counts (clamped to the capacities)
+__global__ void __launch_bounds__(kFinBlock)
+k_points_finalize(const float* __restrict__ dist1, const float* __restrict__ dist2, const int32_t* __restrict__ n_pred,
+                  uint32_t cap_p, const int32_t* __restrict__ n_gt, uint32_t cap_g, float fscore_threshold,
+                  float* __restrict__ row) {
+    __shared__ double red[kFinBlock / 32];
+    const uint32_t np_ = (uint32_t)min(max(*n_pred, 0), (int32_t)cap_p), ng = (uint32_t)min(max(*n_gt, 0), (int32_t)cap_g);
+    double chamfer, fscore;
+    points_metrics(dist1, dist2, np_, ng, fscore_threshold, red, chamfer, fscore);
+    if (threadIdx.x != 0) return;
+    row[0] = (float)chamfer;
+    row[1] = (float)fscore;
+    row[2] = (float)np_;
+    row[3] = (float)ng;
 }
 
 // ------------------------------------------------------------------------------------------------- camera
@@ -527,6 +553,22 @@ CameraWs camera_ws(uint32_t H, uint32_t W) {
 
 // frames up to 2^26 pixels (a 66 x 1030 LiDAR frame has 67 980, a 376 x 1408 camera frame 529 408)
 bool frame_ok(uint32_t H, uint32_t W) { return H > 0 && W > 0 && (uint64_t)H * W <= (1ull << 26); }
+
+struct PointsWs {
+    size_t ch_ws, d1, d2, i1, i2, bytes;
+};
+
+PointsWs points_ws(uint32_t cap_p, uint32_t cap_g) {
+    Carve c;
+    PointsWs w;
+    w.ch_ws = c.take<unsigned char>(nvsf_chamfer_workspace_bytes(1, cap_p, cap_g));
+    w.d1 = c.take<float>(cap_p);
+    w.d2 = c.take<float>(cap_g);
+    w.i1 = c.take<int32_t>(cap_p);
+    w.i2 = c.take<int32_t>(cap_g);
+    w.bytes = c.off;
+    return w;
+}
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
@@ -626,6 +668,32 @@ int nvsf_eval_lidar(const float* depth, const float* image, const float* gt, uin
     if (st != NVSF_OK) return st;
     k_lidar_finalize<<<1, kFinBlock, 0, s>>>(stats, ssim_part, sg, sel, n, max_depth, fscore_threshold, d1, d2,
                                              counts, row);
+    return nvsf_launch_status();
+}
+
+size_t nvsf_eval_points_workspace_bytes(uint32_t cap_p, uint32_t cap_g) {
+    if (cap_p == 0 || cap_g == 0 || cap_p > INT32_MAX || cap_g > INT32_MAX) return 0;
+    return points_ws(cap_p, cap_g).bytes;
+}
+
+int nvsf_eval_points(const float* pred, uint32_t cap_p, const int32_t* n_pred, const float* gt, uint32_t cap_g,
+                     const int32_t* n_gt, float fscore_threshold, float* row, void* workspace, size_t workspace_bytes,
+                     void* stream) {
+    if (!pred || !n_pred || !gt || !n_gt || !row || !workspace || !aligned16(workspace)) return NVSF_E_INVALID;
+    if (cap_p == 0 || cap_g == 0 || cap_p > INT32_MAX || cap_g > INT32_MAX || !(fscore_threshold >= 0.f))
+        return NVSF_E_INVALID;
+    if (workspace_bytes < nvsf_eval_points_workspace_bytes(cap_p, cap_g)) return NVSF_E_WORKSPACE;
+    const PointsWs w = points_ws(cap_p, cap_g);
+    char* base = reinterpret_cast<char*>(workspace);
+    float* d1 = reinterpret_cast<float*>(base + w.d1);
+    float* d2 = reinterpret_cast<float*>(base + w.d2);
+    const int st = nvsf_chamfer_forward_counted(pred, gt, cap_p, cap_g, n_pred, n_gt, d1, d2,
+                                                reinterpret_cast<int32_t*>(base + w.i1),
+                                                reinterpret_cast<int32_t*>(base + w.i2), base + w.ch_ws,
+                                                nvsf_chamfer_workspace_bytes(1, cap_p, cap_g), stream);
+    if (st != NVSF_OK) return st;
+    k_points_finalize<<<1, kFinBlock, 0, (cudaStream_t)stream>>>(d1, d2, n_pred, cap_p, n_gt, cap_g, fscore_threshold,
+                                                                 row);
     return nvsf_launch_status();
 }
 

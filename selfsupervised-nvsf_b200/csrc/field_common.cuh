@@ -189,6 +189,8 @@ int nvsf_train_set_option(const char* name, int value);  // train.cu
 int nvsf_train_get_option(const char* name);
 int nvsf_render_set_option(const char* name, int value);  // render.cu
 int nvsf_render_get_option(const char* name);
+int nvsf_chamfer_set_option(const char* name, int value);  // chamfer.cu
+int nvsf_chamfer_get_option(const char* name);
 int nvsf_heads_tc();                                    // render.cu: option "heads_tc"
 // Compositing + heads launcher (render.cu); scratch = sigma f32 [N*S] then geo f16 [N*S,16];
 // rgbs (f32 [N*S,4], may be NULL) receives the per-sample colours for the backward pass.

@@ -1438,10 +1438,10 @@ int nvsf_render_set_option(const char* name, int value) {
         g_heads_tc = value;
         return NVSF_OK;
     }
-    return NVSF_E_INVALID;
+    return nvsf_chamfer_set_option(name, value);
 }
 int nvsf_heads_tc() { return g_heads_tc; }
 int nvsf_render_get_option(const char* name) {
     if (std::string(name) == "heads_tc") return g_heads_tc;
-    return NVSF_E_INVALID;
+    return nvsf_chamfer_get_option(name);
 }

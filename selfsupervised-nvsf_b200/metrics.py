@@ -21,6 +21,7 @@ LIDAR_METRICS = ("depth_rmse", "depth_medae", "depth_psnr", "depth_ssim",
                  "raydrop_rmse", "raydrop_acc", "raydrop_f1",
                  "chamfer", "fscore", "points_pred", "points_gt")
 CAMERA_METRICS = ("psnr", "ssim")
+POINTS_METRICS = ("chamfer", "fscore", "points_pred", "points_gt")
 
 
 def _frame(t, H, W, C, what):
@@ -159,15 +160,17 @@ def summarize(rows, names, process_group=None):
 class _Meter:
     names = ()
 
-    def __init__(self, H, W, ws_bytes_fn, device):
-        self.H, self.W = int(H), int(W)
+    def __init__(self, device):
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        self._rows = []
+
+    def _frame_workspace(self, H, W, ws_bytes_fn):
+        self.H, self.W = int(H), int(W)
         wb = ws_bytes_fn(self.H, self.W) if self.H > 0 and self.W > 0 else 0
         if wb == 0:
             raise NvsfError(f"{type(self).__name__}: frame {H}x{W} out of range")
         # one workspace for every update: updates of one meter run in one stream, one after another
         self._ws = torch.empty(wb, dtype=torch.uint8, device=self.device)
-        self._rows = []
 
     def _new_row(self):
         row = torch.empty(len(self.names), dtype=torch.float32, device=self.device)
@@ -196,7 +199,8 @@ class LidarMeter(_Meter):
     names = LIDAR_METRICS
 
     def __init__(self, H, W, intrinsics, intrinsics_hoz, scale, max_depth=80.0, fscore_threshold=0.05, device=None):
-        super().__init__(H, W, _lib.lib().nvsf_eval_lidar_workspace_bytes, device)
+        super().__init__(device)
+        self._frame_workspace(H, W, _lib.lib().nvsf_eval_lidar_workspace_bytes)
         self.fovs = _fovs(intrinsics, intrinsics_hoz)
         self.scale, self.max_depth, self.fscore_threshold = float(scale), float(max_depth), float(fscore_threshold)
 
@@ -226,7 +230,8 @@ class CameraMeter(_Meter):
     names = CAMERA_METRICS
 
     def __init__(self, H, W, device=None):
-        super().__init__(H, W, _lib.lib().nvsf_eval_camera_workspace_bytes, device)
+        super().__init__(device)
+        self._frame_workspace(H, W, _lib.lib().nvsf_eval_camera_workspace_bytes)
 
     @torch.no_grad()
     @_lib.device_guard
@@ -239,4 +244,53 @@ class CameraMeter(_Meter):
         row = self._new_row()
         check(_lib.lib().nvsf_eval_camera(ptr(p), ptr(g), self.H, self.W, ptr(row), ptr(self._ws), self._ws.numel(),
                                           stream_ptr()), "CameraMeter.update")
+        return row
+
+
+class PointsMeter(_Meter):
+    """LidarMeter's point metrics for arbitrary clouds (DESIGN.md §3.5): the Chamfer distance (mean squared
+    nearest-neighbour distance, both ways), the F-score of the squared distances below `fscore_threshold` and the
+    two point counts, of a predicted vs a ground-truth cloud of any size: raw scans, accumulated clouds,
+    `lidar_points` outputs.  (+inf, 0) when a cloud is empty."""
+    names = POINTS_METRICS
+
+    def __init__(self, fscore_threshold=0.05, device=None):
+        super().__init__(device)
+        self.fscore_threshold = float(fscore_threshold)
+
+    def _cloud(self, pts, count, what):
+        if not torch.is_tensor(pts) or not pts.is_cuda:
+            raise NvsfError(f"PointsMeter {what}: GPU tensors only")
+        if pts.device != self.device:
+            raise NvsfError(f"PointsMeter: inputs must be on {self.device}")
+        if pts.dtype != torch.float32 or pts.dim() != 2 or pts.shape[1] not in (3, 4):
+            raise NvsfError(f"PointsMeter {what}: points must be fp32 [P, 3|4], got {pts.dtype} {tuple(pts.shape)}")
+        P = int(pts.shape[0])
+        if P > 2**31 - 1:
+            raise NvsfError(f"PointsMeter {what}: {P} points (at most 2^31 - 1)")
+        if count is not None and (not torch.is_tensor(count) or count.device != self.device or count.numel() != 1):
+            raise NvsfError(f"PointsMeter {what}: the count must be a one-element tensor on {self.device}")
+        if P == 0:   # the C ABI takes a capacity of at least one row: one padding row, count 0
+            return (torch.zeros(1, 3, dtype=torch.float32, device=self.device), 1,
+                    torch.zeros((), dtype=torch.int32, device=self.device))
+        xyz = pts[:, :3].contiguous()
+        cnt = torch.full((), P, dtype=torch.int32, device=self.device) if count is None else \
+            count.reshape(()).to(torch.int32)
+        return xyz, P, cnt
+
+    @torch.no_grad()
+    @_lib.device_guard
+    def update(self, pred_points, gt_points, pred_count=None, gt_count=None):
+        """Score one pair of clouds: pred_points [P,3|4], gt_points [G,3|4] CUDA fp32 (only xyz is read); the
+        counts are device int32 scalars (as `lidar_points` returns them; None = every row), the rows past a
+        count are ignored.  Enqueues the work in the current stream, stores the row and returns it ([4] device
+        tensor); no host synchronisation."""
+        p, cap_p, n_p = self._cloud(pred_points, pred_count, "pred_points")
+        g, cap_g, n_g = self._cloud(gt_points, gt_count, "gt_points")
+        L = _lib.lib()
+        wb = L.nvsf_eval_points_workspace_bytes(cap_p, cap_g)
+        ws = torch.empty(wb, dtype=torch.uint8, device=self.device)
+        row = self._new_row()
+        check(L.nvsf_eval_points(ptr(p), cap_p, ptr(n_p), ptr(g), cap_g, ptr(n_g), self.fscore_threshold, ptr(row),
+                                 ptr(ws), wb, stream_ptr()), "PointsMeter.update")
         return row
