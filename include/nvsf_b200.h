@@ -33,7 +33,7 @@ extern "C" {
 #define NVSF_E_WORKSPACE (-2) /* workspace too small */
 
 /* ABI version of this header; bumped on any signature change. */
-#define NVSF_B200_ABI_VERSION 18
+#define NVSF_B200_ABI_VERSION 19
 int nvsf_abi_version(void);
 /* Human-readable text for a status returned by any nvsf_* call. */
 const char* nvsf_status_string(int status);
@@ -478,6 +478,60 @@ size_t nvsf_grid_update_workspace_bytes(uint32_t n);
 int nvsf_grid_update(float* density_grid, const float* tmp_grid, uint32_t n, float decay,
                      float density_thresh, uint8_t* bitfield, float* stats, void* workspace,
                      size_t workspace_bytes, void* stream);
+
+/* Cells no training sensor sees (torch-ngp's mark_untrained_grid; contract in DESIGN.md §3.5).
+ *
+ * nvsf_grid_coverage_camera / _lidar: OR into `covered` (C*H^3/8 bytes, [C][Morton] order like the
+ *   bitfield, 4-byte aligned, C*H^3 a multiple of 32) the cells whose un-jittered centre x (the
+ *   noise = NULL point of nvsf_grid_cell_points) some pose of poses [B,4,4] (sensor-to-world, row-major,
+ *   device fp32) sees, with margin m = fl(2 b_c / H).  p = R^T (x - t), every product and sum rounded on
+ *   its own: d_b = x_b - t_b, p_a = (R[0][a] d_0 + R[1][a] d_1) + R[2][a] d_2.
+ *   Camera (x right, y down, z forward, image img_H x img_W): p.z > 0, fl(sl p.z) - m < p.x <
+ *   fl(sr p.z) + m and fl(st p.z) - m < p.y < fl(sb p.z) + m with sl = -cx/fx, sr = (img_W - cx)/fx,
+ *   st = -cy/fy, sb = (img_H - cy)/fy.
+ *   LiDAR (degrees; range [near, far]): with r = sqrt((p.x^2 + p.y^2) + p.z^2) and rho = sqrt(p.x^2 +
+ *   p.y^2), fl(near - m) < r < fl(far + m) and fl(s_lo rho) - m < p.z < fl(s_up rho) + m, s_up =
+ *   tan(fov_up), s_lo = tan(fov_up - fov); below fov_hoz = 360 also n1.p > -m and / or (fov_hoz > 180)
+ *   n2.p > -m with n1 = (sin h, cos h), n2 = (sin h, -cos h), h = fov_hoz / 2, n.p = fl(n.x p.x) +
+ *   fl(n.y p.y).  Slopes and normals are computed in float64 and rounded to fp32 once.  NVSF_E_INVALID
+ *   for fov_up >= 90, fov_up - fov <= -90, fov <= 0, fov_hoz outside (0, 360], near < 0 or far <= near;
+ *   for fx, fy <= 0 or a non-finite camera intrinsic.  B == 0 is a no-op.
+ * nvsf_grid_apply_marks: density_grid = -1 and bitfield bit cleared where the cell is not covered; a
+ *   covered cell holding a mark (< 0) becomes 0.  *n_marked (device int32) = number of uncovered cells.
+ *   n = C*H^3, a multiple of 8.  stats are untouched until the next update. */
+int nvsf_grid_coverage_camera(uint32_t C, uint32_t H, float bound, const float* poses, uint32_t B, float fx,
+                              float fy, float cx, float cy, uint32_t img_H, uint32_t img_W, uint8_t* covered,
+                              void* stream);
+int nvsf_grid_coverage_lidar(uint32_t C, uint32_t H, float bound, const float* poses, uint32_t B, float fov_up,
+                             float fov, float fov_hoz, float near, float far, uint8_t* covered, void* stream);
+int nvsf_grid_apply_marks(float* density_grid, uint8_t* bitfield, const uint8_t* covered, uint32_t n,
+                          int32_t* n_marked, void* stream);
+
+/* Cell lists for updates that skip marked cells and for torch-ngp's partial update.
+ *
+ * nvsf_grid_cell_list: cells [<= C*H3] (int32 ids c*H3 + m, ascending) = the cells with grid >= 0
+ *   (above = 0: the trainable cells) or grid > 0 (above = 1: the occupied cells); offsets [C+1] (device
+ *   int32): offsets[c] = list position of cascade c's first listed cell, offsets[C] = list length.
+ *   Order-preserving, no atomics; workspace nvsf_grid_cell_list_workspace_bytes(C*H3).
+ * nvsf_grid_cell_points_list: xyz [count,3] = nvsf_grid_cell_points' point of each listed cell (the origin
+ *   for a negative id), jitter row noise[cells[r]] (noise_by_cell != 0) or noise[r]; noise NULL = centres.
+ * nvsf_grid_draws: cells [C * H3/2] of the partial update.  Per cascade c, slot s < Q = H3/4 draws a cell
+ *   of the cascade uniformly, slot Q <= s < 2Q one of its occupied cells uniformly (the offsets / occupied
+ *   list of nvsf_grid_cell_list with above = 1; -1 when the cascade has none).  The draw is the high 32
+ *   bits hi of h = splitmix64(k ^ (c << 32 | s)), k = splitmix64(splitmix64(seed) ^ iter), reduced to
+ *   [0, range) as (hi * range) >> 32.  H3 a multiple of 4.
+ * nvsf_grid_scatter_max: tmp_grid[cells[r]] = max(tmp_grid[cells[r]], vals[r]) for 0 <= cells[r] < n, by
+ *   the ordering of the values' bits as int32 (exact for tmp = -1 and vals >= 0; a cell drawn twice keeps
+ *   the maximum whatever the order). */
+size_t nvsf_grid_cell_list_workspace_bytes(uint32_t n);
+int nvsf_grid_cell_list(const float* density_grid, uint32_t C, uint32_t H3, uint32_t above, int32_t* cells,
+                        int32_t* offsets, void* workspace, size_t workspace_bytes, void* stream);
+int nvsf_grid_cell_points_list(uint32_t C, uint32_t H, float bound, const int32_t* cells, uint32_t count,
+                               const float* noise, uint32_t noise_by_cell, float* xyz, void* stream);
+int nvsf_grid_draws(uint32_t C, uint32_t H3, uint64_t seed, uint64_t iter, const int32_t* occupied,
+                    const int32_t* offsets, int32_t* cells, void* stream);
+int nvsf_grid_scatter_max(float* tmp_grid, uint32_t n, const int32_t* cells, const float* vals, uint32_t count,
+                          void* stream);
 
 /* Order-preserving compaction out = rays_alive[rays_alive >= 0] of the inference loop around
  * march_rays / composite_rays (composite_rays marks finished rays with -1, raymarching.cu:1049);

@@ -103,6 +103,14 @@ PROTOTYPES = {
     "nvsf_grid_accumulate": (_int, [_p, _p, _u32, _f32, _u32, _p]),
     "nvsf_grid_update_workspace_bytes": (_sz, [_u32]),
     "nvsf_grid_update": (_int, [_p, _p, _u32, _f32, _f32, _p, _p, _p, _sz, _p]),
+    "nvsf_grid_coverage_camera": (_int, [_u32, _u32, _f32, _p, _u32, _f32, _f32, _f32, _f32, _u32, _u32, _p, _p]),
+    "nvsf_grid_coverage_lidar": (_int, [_u32, _u32, _f32, _p, _u32, _f32, _f32, _f32, _f32, _f32, _p, _p]),
+    "nvsf_grid_apply_marks": (_int, [_p, _p, _p, _u32, _p, _p]),
+    "nvsf_grid_cell_list_workspace_bytes": (_sz, [_u32]),
+    "nvsf_grid_cell_list": (_int, [_p, _u32, _u32, _u32, _p, _p, _p, _sz, _p]),
+    "nvsf_grid_cell_points_list": (_int, [_u32, _u32, _f32, _p, _u32, _p, _u32, _p, _p]),
+    "nvsf_grid_draws": (_int, [_u32, _u32, ctypes.c_uint64, ctypes.c_uint64, _p, _p, _p, _p]),
+    "nvsf_grid_scatter_max": (_int, [_p, _u32, _p, _p, _u32, _p]),
     "nvsf_compact_alive_workspace_bytes": (_sz, [_u32]),
     "nvsf_compact_alive": (_int, [_p, _u32, _p, _p, _p, _sz, _p]),
     # Part 5 — loss head
@@ -164,7 +172,7 @@ def lib():
     return _lib
 
 
-ABI_VERSION = 18
+ABI_VERSION = 19
 
 
 def check(status, what=""):

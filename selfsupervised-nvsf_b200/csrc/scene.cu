@@ -12,6 +12,7 @@
 //    grid = max(grid * decay, new) on valid cells, threshold = min(mean(clamp(grid, 0)),
 //    density_thresh), packbits.  Mean, threshold and packing stay on the device (no host sync).
 #include <algorithm>
+#include <cmath>
 
 #include "common.cuh"
 #include "lidar_dir.cuh"
@@ -173,13 +174,10 @@ __device__ __forceinline__ uint32_t compact_by3(uint32_t x) {  // raymarching.cu
 // i.e. already in the [C, H^3] Morton layout of the density grid.
 // `first` / `count` select a slice of the C*H^3 cells (multi-GPU update: each rank owns one slice);
 // noise and xyz rows are relative to the slice.
-__global__ void __launch_bounds__(256)
-k_grid_cell_points(uint32_t C, uint32_t H, float bound, const float* __restrict__ noise,
-                   float* __restrict__ xyz, size_t first, size_t count) {
+// Sample point of cell g = c*H^3 + m; `noise` points at the cell's 3 jitter values or is NULL.
+__device__ __forceinline__ void cell_point(size_t g, uint32_t H, float bound, const float* __restrict__ noise,
+                                           float v[3]) {
     const uint32_t H3 = H * H * H;
-    const size_t r = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= count) return;
-    const size_t g = first + r;
     const uint32_t c = (uint32_t)(g / H3), m = (uint32_t)(g % H3);
     const float bc = fminf(exp2f((float)c), bound);
     const float half = __fdiv_rn(bc, (float)H);
@@ -188,13 +186,214 @@ k_grid_cell_points(uint32_t C, uint32_t H, float bound, const float* __restrict_
 #pragma unroll
     for (int a = 0; a < 3; ++a) {
         const float u = __fsub_rn(__fdiv_rn(__fmul_rn(2.0f, (float)co[a]), (float)(H - 1)), 1.0f);
-        float v = __fmul_rn(u, ext);
+        v[a] = __fmul_rn(u, ext);
         if (noise) {
-            const float j = __fsub_rn(__fmul_rn(__ldg(noise + r * 3 + a), 2.0f), 1.0f);
-            v = __fadd_rn(v, __fmul_rn(j, half));
+            const float j = __fsub_rn(__fmul_rn(__ldg(noise + a), 2.0f), 1.0f);
+            v[a] = __fadd_rn(v[a], __fmul_rn(j, half));
         }
-        xyz[r * 3 + a] = v;
     }
+}
+
+__global__ void __launch_bounds__(256)
+k_grid_cell_points(uint32_t C, uint32_t H, float bound, const float* __restrict__ noise,
+                   float* __restrict__ xyz, size_t first, size_t count) {
+    const size_t r = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= count) return;
+    float v[3];
+    cell_point(first + r, H, bound, noise ? noise + r * 3 : nullptr, v);
+#pragma unroll
+    for (int a = 0; a < 3; ++a) xyz[r * 3 + a] = v[a];
+}
+
+// Sample points of the cells listed in cells[0, count) (ids c*H^3 + m; a negative id yields the origin).
+// The jitter row of entry r is noise[cells[r]] when noise_by_cell, else noise[r].
+__global__ void __launch_bounds__(256)
+k_grid_cell_points_list(uint32_t H, float bound, const int32_t* __restrict__ cells, uint32_t count,
+                        const float* __restrict__ noise, uint32_t noise_by_cell, float* __restrict__ xyz) {
+    const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= count) return;
+    const int32_t g = __ldg(cells + r);
+    float v[3] = {0.f, 0.f, 0.f};
+    if (g >= 0) cell_point((size_t)g, H, bound, noise ? noise + (size_t)(noise_by_cell ? (uint32_t)g : r) * 3 : nullptr,
+                           v);
+#pragma unroll
+    for (int a = 0; a < 3; ++a) xyz[(size_t)r * 3 + a] = v[a];
+}
+
+// --------------------------------------------------------------------------- untrained-cell marking
+// torch-ngp's mark_untrained_grid with the tests of DESIGN.md §3.5: a cell is covered by a pose when its
+// un-jittered centre lies inside the sensor's field of view widened by the margin m = 2 b_c / H.  Every
+// slope and edge normal is prepared on the host in float64 and rounded to fp32 once; the kernel only
+// multiplies, adds and compares, each operation rounded on its own, so a numpy fp32 restatement gives
+// the same bits.
+constexpr uint32_t kCovPoses = 128;  // poses per launch, kept in shared memory (12 floats each)
+
+struct Coverage {
+    uint32_t lidar;  // 0: camera frustum, 1: LiDAR shell
+    // camera: x-slopes (sl, sr), y-slopes (st, sb); LiDAR: range [near, far], elevation slopes (s_lo, s_up)
+    float a0, a1, a2, a3;
+    uint32_t wedge;  // LiDAR azimuth: 0 none (360 degrees), 1 intersection of the two half-planes, 2 union
+    float n1x, n1y, n2x, n2y;
+};
+
+__device__ __forceinline__ bool covers(const Coverage& S, const float* P, const float x[3], float m) {
+    // p = R^T (x - t): d_b = fl(x_b - t_b), p_a = fl(fl(fl(R[0][a] d_0) + fl(R[1][a] d_1)) + fl(R[2][a] d_2))
+    const float d0 = __fsub_rn(x[0], P[3]), d1 = __fsub_rn(x[1], P[7]), d2 = __fsub_rn(x[2], P[11]);
+    float p[3];
+#pragma unroll
+    for (int a = 0; a < 3; ++a)
+        p[a] = __fadd_rn(__fadd_rn(__fmul_rn(P[a], d0), __fmul_rn(P[4 + a], d1)), __fmul_rn(P[8 + a], d2));
+    if (!S.lidar) {
+        if (!(p[2] > 0.f)) return false;
+        if (!(p[0] > __fsub_rn(__fmul_rn(S.a0, p[2]), m) && p[0] < __fadd_rn(__fmul_rn(S.a1, p[2]), m))) return false;
+        return p[1] > __fsub_rn(__fmul_rn(S.a2, p[2]), m) && p[1] < __fadd_rn(__fmul_rn(S.a3, p[2]), m);
+    }
+    const float xy = __fadd_rn(__fmul_rn(p[0], p[0]), __fmul_rn(p[1], p[1]));
+    const float r = __fsqrt_rn(__fadd_rn(xy, __fmul_rn(p[2], p[2])));
+    const float rho = __fsqrt_rn(xy);
+    if (!(r > __fsub_rn(S.a0, m) && r < __fadd_rn(S.a1, m))) return false;
+    if (!(p[2] > __fsub_rn(__fmul_rn(S.a2, rho), m) && p[2] < __fadd_rn(__fmul_rn(S.a3, rho), m))) return false;
+    if (S.wedge == 0) return true;
+    const bool in1 = __fadd_rn(__fmul_rn(S.n1x, p[0]), __fmul_rn(S.n1y, p[1])) > -m;
+    const bool in2 = __fadd_rn(__fmul_rn(S.n2x, p[0]), __fmul_rn(S.n2y, p[1])) > -m;
+    return S.wedge == 1 ? (in1 && in2) : (in1 || in2);
+}
+
+// One thread per cell; a warp owns one 32-bit word of the covered mask (bit i of byte k = cell 8k + i) and
+// ORs its ballot into it.  Cells already covered skip the poses; a cell stops at its first covering pose.
+__global__ void __launch_bounds__(256)
+k_grid_coverage(uint32_t n, uint32_t H, float bound, const float* __restrict__ poses, uint32_t B, Coverage S,
+                uint32_t* __restrict__ covered) {
+    __shared__ float P[kCovPoses * 12];
+    for (uint32_t i = threadIdx.x; i < B * 12; i += blockDim.x) P[i] = __ldg(poses + (i / 12) * 16 + i % 12);
+    __syncthreads();
+    const uint32_t g = blockIdx.x * blockDim.x + threadIdx.x;  // n is a multiple of 32: whole warps
+    if (g >= n) return;
+    const uint32_t lane = threadIdx.x & 31, word = covered[g >> 5];
+    bool cov = (word >> lane) & 1u;
+    if (!cov) {
+        const uint32_t H3 = H * H * H;
+        const float bc = fminf(exp2f((float)(g / H3)), bound);
+        const float m = __fdiv_rn(__fmul_rn(2.0f, bc), (float)H);
+        float x[3];
+        cell_point(g, H, bound, nullptr, x);
+        for (uint32_t b = 0; b < B && !cov; ++b) cov = covers(S, P + b * 12, x, m);
+    }
+    const uint32_t bal = __ballot_sync(0xffffffffu, cov);
+    if (lane == 0 && bal != word) covered[g >> 5] = bal;
+}
+
+// Applies the covered mask, one thread per mask byte (8 cells): uncovered cells get grid = -1 and their
+// bitfield bit cleared; a covered cell that holds a mark from an earlier call is restored to 0.
+// *n_marked (zeroed by the caller) receives the number of uncovered cells.
+__global__ void __launch_bounds__(256)
+k_grid_apply_marks(float* __restrict__ grid, uint8_t* __restrict__ bitfield, const uint8_t* __restrict__ covered,
+                   uint32_t n_bytes, int32_t* __restrict__ n_marked) {
+    const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
+    uint32_t marked = 0;
+    if (b < n_bytes) {
+        const uint32_t cov = covered[b];
+        marked = 8u - __popc(cov);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            float* g = grid + (size_t)b * 8 + i;
+            if (!((cov >> i) & 1u)) *g = -1.f;
+            else if (*g < 0.f) *g = 0.f;
+        }
+        bitfield[b] &= (uint8_t)cov;
+    }
+    marked = warp_reduce_sum(marked);
+    if ((threadIdx.x & 31) == 0 && marked) atomicAdd(n_marked, (int32_t)marked);
+}
+
+// Order-preserving list of the cells with grid >= 0 (above = 0) or grid > 0 (above = 1), as int32 cell ids,
+// by per-CTA counts then a scatter (like the alive-list compaction).  offsets[c] (c < C) receives the list
+// position of the first listed cell of cascade c and offsets[C] the length: the list is cascade-major.
+constexpr int kCellBlock = 1024;
+__device__ __forceinline__ bool cell_listed(const float* grid, uint32_t i, uint32_t n, uint32_t above) {
+    if (i >= n) return false;
+    const float g = grid[i];
+    return above ? g > 0.f : g >= 0.f;
+}
+
+__global__ void __launch_bounds__(kCellBlock)
+k_cell_count(const float* __restrict__ grid, uint32_t n, uint32_t above, uint32_t* __restrict__ counts) {
+    const uint32_t c = __syncthreads_count(cell_listed(grid, blockIdx.x * kCellBlock + threadIdx.x, n, above));
+    if (threadIdx.x == 0) counts[blockIdx.x] = c;
+}
+
+__global__ void __launch_bounds__(kCellBlock)
+k_cell_scatter(const float* __restrict__ grid, uint32_t n, uint32_t H3, uint32_t above,
+               const uint32_t* __restrict__ counts, int32_t* __restrict__ out, int32_t* __restrict__ offsets) {
+    __shared__ uint32_t warp_off[kCellBlock / 32 + 1];
+    __shared__ uint32_t base_s;
+    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (tid < 32) {  // exclusive prefix of the CTA counts before this CTA
+        uint32_t s = 0;
+        for (uint32_t b = lane; b < blockIdx.x; b += 32) s += counts[b];
+        s = warp_reduce_sum(s);
+        if (lane == 0) base_s = s;
+    }
+    const uint32_t i = blockIdx.x * kCellBlock + tid;
+    const bool keep = cell_listed(grid, i, n, above);
+    const uint32_t bal = __ballot_sync(0xffffffffu, keep);
+    if (lane == 0) warp_off[warp] = __popc(bal);
+    __syncthreads();
+    if (tid < 32) {
+        const uint32_t c = warp_off[tid];
+        const uint32_t inc = warp_inclusive_scan(c, lane);
+        warp_off[tid] = inc - c;
+        if (tid == 31) warp_off[kCellBlock / 32] = inc;
+    }
+    __syncthreads();
+    const uint32_t pos = base_s + warp_off[warp] + __popc(bal & ((1u << lane) - 1u));
+    if (keep) out[pos] = (int32_t)i;
+    if (i < n && i % H3 == 0) offsets[i / H3] = (int32_t)pos;
+    if (tid == 0 && blockIdx.x == gridDim.x - 1) offsets[n / H3] = (int32_t)(base_s + warp_off[kCellBlock / 32]);
+}
+
+// ------------------------------------------------------------------------------ partial update draws
+// torch-ngp's partial update: per cascade c, slots s < Q = H^3/4 draw a uniformly random cell of the cascade,
+// slots Q <= s < 2Q draw uniformly from the cascade's ascending list of cells with grid > 0 (slot -> -1 when
+// that list is empty).  The draw of (seed, iter, c, s) is the high 32 bits of
+// h = splitmix64(splitmix64(splitmix64(seed) ^ iter) ^ (c << 32 | s)) reduced to [0, range) as (hi * range) >> 32.
+__host__ __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
+    uint64_t z = x + 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+
+__global__ void __launch_bounds__(256)
+k_grid_draws(uint32_t C, uint32_t H3, uint64_t key, const int32_t* __restrict__ occupied,
+             const int32_t* __restrict__ offsets, int32_t* __restrict__ cells) {
+    const uint32_t Q = H3 / 4, D = 2 * Q;
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= C * D) return;
+    const uint32_t c = k / D, s = k % D;
+    const uint64_t h = splitmix64(key ^ ((uint64_t)c << 32 | s));
+    const uint64_t hi = h >> 32;
+    int32_t cell;
+    if (s < Q) {
+        cell = (int32_t)(c * H3 + (uint32_t)((hi * H3) >> 32));
+    } else {
+        const int32_t lo = __ldg(offsets + c), cnt = __ldg(offsets + c + 1) - lo;
+        cell = cnt > 0 ? __ldg(occupied + lo + (uint32_t)((hi * (uint32_t)cnt) >> 32)) : -1;
+    }
+    cells[k] = cell;
+}
+
+// tmp[cells[r]] = max(tmp[cells[r]], vals[r]) for cells[r] >= 0.  tmp starts at -1 and the values are
+// sigma * density_scale >= 0, whose order is that of their bit patterns as signed integers: an integer
+// atomicMax keeps the maximum whatever the order of the writes (a negative value leaves the cell alone).
+__global__ void __launch_bounds__(256)
+k_grid_scatter_max(float* __restrict__ tmp, const int32_t* __restrict__ cells, const float* __restrict__ vals,
+                   uint32_t count, uint32_t n) {
+    const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= count) return;
+    const int32_t g = __ldg(cells + r);
+    if (g < 0 || (uint32_t)g >= n) return;
+    atomicMax(reinterpret_cast<int*>(tmp) + g, __float_as_int(__ldg(vals + r)));
 }
 
 // tmp = sigma * density_scale (first pass) or max(tmp, sigma * density_scale) (further times)
@@ -399,6 +598,125 @@ int nvsf_grid_update(float* density_grid, const float* tmp_grid, uint32_t n, flo
     k_grid_update<<<nblk, kUpdBlock, 0, s>>>(density_grid, tmp_grid, n, decay, partial);
     k_grid_stats<<<1, 32, 0, s>>>(partial, nblk, n, density_thresh, stats);
     k_packbits_dev<<<nvsf_div_up(n / 8, 256u), 256, 0, s>>>(density_grid, n / 8, stats, bitfield);
+    return nvsf_launch_status();
+}
+
+int nvsf_grid_cell_points_list(uint32_t C, uint32_t H, float bound, const int32_t* cells, uint32_t count,
+                               const float* noise, uint32_t noise_by_cell, float* xyz, void* stream) {
+    if (C == 0 || H < 2 || H > 1024 || !(bound > 0.f) || (uint64_t)C * H * H * H > INT32_MAX) return NVSF_E_INVALID;
+    if (count == 0) return NVSF_OK;
+    if (!cells || !xyz) return NVSF_E_INVALID;
+    k_grid_cell_points_list<<<nvsf_div_up(count, 256u), 256, 0, (cudaStream_t)stream>>>(H, bound, cells, count,
+                                                                                        noise, noise_by_cell, xyz);
+    return nvsf_launch_status();
+}
+
+// Checks shared by the coverage entry points; n = C*H^3 must fill whole 32-bit mask words.
+static bool coverage_args_ok(uint32_t C, uint32_t H, float bound, const float* poses, uint8_t* covered) {
+    if (!poses || !covered || C == 0 || H < 2 || H > 1024 || !(bound > 0.f)) return false;
+    const uint64_t n = (uint64_t)C * H * H * H;
+    return n % 32 == 0 && n <= INT32_MAX && (reinterpret_cast<uintptr_t>(covered) & 3) == 0;
+}
+
+static int launch_coverage(uint32_t C, uint32_t H, float bound, const float* poses, uint32_t B, const Coverage& S,
+                           uint8_t* covered, cudaStream_t s) {
+    const uint32_t n = C * H * H * H;
+    for (uint32_t b0 = 0; b0 < B; b0 += kCovPoses) {
+        k_grid_coverage<<<nvsf_div_up(n, 256u), 256, 0, s>>>(n, H, bound, poses + (size_t)b0 * 16,
+                                                             std::min(kCovPoses, B - b0), S,
+                                                             reinterpret_cast<uint32_t*>(covered));
+        const int e = nvsf_launch_status();
+        if (e != NVSF_OK) return e;
+    }
+    return NVSF_OK;
+}
+
+int nvsf_grid_coverage_camera(uint32_t C, uint32_t H, float bound, const float* poses, uint32_t B, float fx,
+                              float fy, float cx, float cy, uint32_t img_H, uint32_t img_W, uint8_t* covered,
+                              void* stream) {
+    if (B == 0) return NVSF_OK;
+    if (!coverage_args_ok(C, H, bound, poses, covered) || img_H == 0 || img_W == 0) return NVSF_E_INVALID;
+    if (!(fx > 0.f) || !(fy > 0.f) || !std::isfinite(fx) || !std::isfinite(fy) || !std::isfinite(cx) ||
+        !std::isfinite(cy))
+        return NVSF_E_INVALID;
+    Coverage S{};
+    S.lidar = 0;
+    S.a0 = (float)(-(double)cx / (double)fx);
+    S.a1 = (float)(((double)img_W - (double)cx) / (double)fx);
+    S.a2 = (float)(-(double)cy / (double)fy);
+    S.a3 = (float)(((double)img_H - (double)cy) / (double)fy);
+    return launch_coverage(C, H, bound, poses, B, S, covered, (cudaStream_t)stream);
+}
+
+int nvsf_grid_coverage_lidar(uint32_t C, uint32_t H, float bound, const float* poses, uint32_t B, float fov_up,
+                             float fov, float fov_hoz, float near, float far, uint8_t* covered, void* stream) {
+    if (B == 0) return NVSF_OK;
+    if (!coverage_args_ok(C, H, bound, poses, covered)) return NVSF_E_INVALID;
+    const double up = fov_up, lo = (double)fov_up - (double)fov, hoz = fov_hoz;
+    if (!(up < 90.0) || !(lo > -90.0) || !(fov > 0.f) || !(hoz > 0.0 && hoz <= 360.0)) return NVSF_E_INVALID;
+    if (!(near >= 0.f) || !(far > near) || !std::isfinite(far)) return NVSF_E_INVALID;
+    const double deg = 3.14159265358979323846 / 180.0;
+    Coverage S{};
+    S.lidar = 1;
+    S.a0 = near;
+    S.a1 = far;
+    S.a2 = (float)std::tan(lo * deg);
+    S.a3 = (float)std::tan(up * deg);
+    if (hoz < 360.0) {  // wedge [-h, h] of azimuth: inner normals of its edges at -h and +h
+        const double h = 0.5 * hoz * deg, sh = std::sin(h), ch = std::cos(h);
+        S.wedge = hoz <= 180.0 ? 1u : 2u;
+        S.n1x = (float)sh;
+        S.n1y = (float)ch;
+        S.n2x = (float)sh;
+        S.n2y = (float)-ch;
+    }
+    return launch_coverage(C, H, bound, poses, B, S, covered, (cudaStream_t)stream);
+}
+
+int nvsf_grid_apply_marks(float* density_grid, uint8_t* bitfield, const uint8_t* covered, uint32_t n,
+                          int32_t* n_marked, void* stream) {
+    if (!density_grid || !bitfield || !covered || !n_marked || n == 0 || n % 8 != 0) return NVSF_E_INVALID;
+    cudaStream_t s = (cudaStream_t)stream;
+    const cudaError_t e = cudaMemsetAsync(n_marked, 0, sizeof(int32_t), s);
+    if (e != cudaSuccess) return (int)e;
+    k_grid_apply_marks<<<nvsf_div_up(n / 8, 256u), 256, 0, s>>>(density_grid, bitfield, covered, n / 8, n_marked);
+    return nvsf_launch_status();
+}
+
+size_t nvsf_grid_cell_list_workspace_bytes(uint32_t n) {
+    return (size_t)nvsf_div_up(n, (uint32_t)kCellBlock) * sizeof(uint32_t);
+}
+
+int nvsf_grid_cell_list(const float* density_grid, uint32_t C, uint32_t H3, uint32_t above, int32_t* cells,
+                        int32_t* offsets, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!density_grid || !cells || !offsets || !workspace || C == 0 || H3 == 0 || above > 1) return NVSF_E_INVALID;
+    const uint64_t n64 = (uint64_t)C * H3;
+    if (n64 > INT32_MAX) return NVSF_E_INVALID;
+    const uint32_t n = (uint32_t)n64;
+    if (workspace_bytes < nvsf_grid_cell_list_workspace_bytes(n)) return NVSF_E_WORKSPACE;
+    cudaStream_t s = (cudaStream_t)stream;
+    const uint32_t nblk = nvsf_div_up(n, (uint32_t)kCellBlock);
+    uint32_t* counts = reinterpret_cast<uint32_t*>(workspace);
+    k_cell_count<<<nblk, kCellBlock, 0, s>>>(density_grid, n, above, counts);
+    k_cell_scatter<<<nblk, kCellBlock, 0, s>>>(density_grid, n, H3, above, counts, cells, offsets);
+    return nvsf_launch_status();
+}
+
+int nvsf_grid_draws(uint32_t C, uint32_t H3, uint64_t seed, uint64_t iter, const int32_t* occupied,
+                    const int32_t* offsets, int32_t* cells, void* stream) {
+    if (!occupied || !offsets || !cells || C == 0 || H3 < 4 || H3 % 4 != 0 || (uint64_t)C * H3 > INT32_MAX)
+        return NVSF_E_INVALID;
+    const uint32_t draws = C * (H3 / 2);
+    k_grid_draws<<<nvsf_div_up(draws, 256u), 256, 0, (cudaStream_t)stream>>>(
+        C, H3, splitmix64(splitmix64(seed) ^ iter), occupied, offsets, cells);
+    return nvsf_launch_status();
+}
+
+int nvsf_grid_scatter_max(float* tmp_grid, uint32_t n, const int32_t* cells, const float* vals, uint32_t count,
+                          void* stream) {
+    if (count == 0) return NVSF_OK;
+    if (!tmp_grid || !cells || !vals || n == 0) return NVSF_E_INVALID;
+    k_grid_scatter_max<<<nvsf_div_up(count, 256u), 256, 0, (cudaStream_t)stream>>>(tmp_grid, cells, vals, count, n);
     return nvsf_launch_status();
 }
 

@@ -722,7 +722,7 @@ class NeRFNetwork(nn.Module):
     @_lib.device_guard
     @_lib.with_options
     def update_extra_state(self, time=0.0, cal_lidar_color=False, decay=0.95, perturb=True, noise=None,
-                           process_group=None, shard=None):
+                           process_group=None, shard=None, mode="full", seed=0):
         """Full occupancy-grid update (torch-ngp NeRFRenderer.update_extra_state, the caller the
         reference's morton3D / packbits operators were written for): evaluate sigma at one
         jittered point per cell and cascade, grid = max(grid*decay, sigma*density_scale),
@@ -731,12 +731,24 @@ class NeRFNetwork(nn.Module):
         (one bitfield serves a dynamic scene because march_rays* take no time argument).
         `noise` [C*H^3, 3] in [0,1) optionally supplies the jitter.
 
+        After mark_untrained_grid the full update evaluates only the trainable cells (grid >= 0); `noise`
+        rows are still those of the cells, and the result is bit-identical to evaluating every cell.
+
+        mode="partial" is torch-ngp's partial update: per cascade H^3/4 uniformly drawn cells and H^3/4
+        cells drawn from those with grid > 0 (nvsf_grid_draws: a hash of (seed, iter_density, cascade,
+        slot), the same on every rank); only the drawn cells are decayed and refreshed, a cell drawn twice
+        takes the larger value.  Explicit `noise` is then [C*H^3/2, 3], one row per draw.
+        mode="ngp" is torch-ngp's schedule: full while iter_density < 16, partial after that.
+
         Multi-GPU (SURVEY 8e): with torch.distributed initialised (or `shard=True`) every rank
         evaluates the field on ONE contiguous slice of the C*H^3 cells (dist.cell_slice), the ranks
         all_gather the per-cell sigmas (4 B per cell) and each applies the decay / threshold /
         packbits to the whole grid, so all replicas end with the same grid and bitfield.  `noise`
-        given explicitly is the full [C*H^3, 3] array on every rank (each uses its rows)."""
+        given explicitly is the full [C*H^3, 3] array on every rank (each uses its rows).  The list
+        of trainable cells or of draws is sliced the same way."""
         from . import dist as nd
+        if mode not in ("full", "partial", "ngp"):
+            raise ValueError(f"update_extra_state: mode {mode!r} is not 'full', 'partial' or 'ngp'")
         L = _lib.lib()
         lidar = bool(cal_lidar_color)
         st = self._grid_state(lidar)
@@ -748,6 +760,12 @@ class NeRFNetwork(nn.Module):
             shard = world > 1
         if not shard:
             world, rank = 1, 0
+        if mode == "partial" or (mode == "ngp" and st["iter_density"] >= 16):
+            return self._update_cells(st, self._partial_draws(st, seed), False, time, lidar, decay, perturb, noise,
+                                      process_group, world, rank)
+        if st.get("trainable") is not None:
+            return self._update_cells(st, st["trainable"], True, time, lidar, decay, perturb, noise, process_group,
+                                      world, rank)
         per, lo, hi = nd.cell_slice(n, rank, world)
         cnt = hi - lo
         if noise is None and perturb:
@@ -779,6 +797,169 @@ class NeRFNetwork(nn.Module):
               "grid_update")
         st["iter_density"] += 1
         return st["density_bitfield"]
+
+    def _update_cells(self, st, cells, by_cell, time, lidar, decay, perturb, noise, process_group, world, rank):
+        """update_extra_state over a list of cells (int32 ids): sigma at the listed cells' jittered points,
+        max over the times, scattered into tmp = -1 so that unlisted cells are neither decayed nor refreshed.
+        Ranks evaluate one slice of the list each and all_gather the values.  by_cell: `noise` rows are
+        cell ids ([C*H^3, 3]); otherwise list positions ([len(cells), 3])."""
+        from . import dist as nd
+        L = _lib.lib()
+        dev = self.sigma_net.device
+        C, H = self.cascade, self.grid_size
+        n, m = C * H ** 3, cells.shape[0]
+        per, lo, hi = nd.cell_slice(m, rank, world)
+        cnt = hi - lo
+        if noise is not None:
+            noise = noise.detach().to(device=dev, dtype=torch.float32).contiguous().view(-1, 3)
+            want = n if by_cell else m
+            if noise.shape[0] != want:
+                raise _lib.NvsfError(f"noise has {noise.shape[0]} rows, expected {want} "
+                                     f"({'one per cell' if by_cell else 'one per draw'})")
+            if not by_cell:
+                noise = noise[lo:hi]
+        elif perturb:
+            noise, by_cell = torch.rand(cnt, 3, dtype=torch.float32, device=dev), False
+        xyz = torch.empty(cnt, 3, dtype=torch.float32, device=dev)
+        check(L.nvsf_grid_cell_points_list(C, H, self.bound, ptr(cells[lo:hi]), cnt, ptr(noise), int(by_cell),
+                                           ptr(xyz), stream_ptr()), "grid_cell_points_list")
+        gathered = torch.zeros(world * per, dtype=torch.float32, device=dev) if world > 1 else None
+        vals = gathered[rank * per:rank * per + per] if world > 1 else torch.empty(m, dtype=torch.float32, device=dev)
+        if cnt > 0:
+            times = list(time) if isinstance(time, (list, tuple)) else [time]
+            for k, t in enumerate(times):
+                sigma, _, _, _ = self._density_raw(xyz, t, lidar)
+                check(L.nvsf_grid_accumulate(ptr(vals), ptr(sigma), cnt, self.density_scale, int(k == 0),
+                                             stream_ptr()), "grid_accumulate")
+        if world > 1 and per > 0:
+            import torch.distributed as tdist
+            tdist.all_gather_into_tensor(gathered, vals.clone(), group=process_group)
+            vals = gathered[:m]
+        tmp = torch.full((n,), -1.0, dtype=torch.float32, device=dev)
+        check(L.nvsf_grid_scatter_max(ptr(tmp), n, ptr(cells), ptr(vals), m, stream_ptr()), "grid_scatter_max")
+        wbytes = L.nvsf_grid_update_workspace_bytes(n)
+        ws = torch.empty(wbytes, dtype=torch.uint8, device=dev)
+        check(L.nvsf_grid_update(ptr(st["density_grid"]), ptr(tmp), n, float(decay), float(self.density_thresh),
+                                 ptr(st["density_bitfield"]), ptr(st["stats"]), ptr(ws), wbytes, stream_ptr()),
+              "grid_update")
+        st["iter_density"] += 1
+        return st["density_bitfield"]
+
+    def _cell_list(self, st, above):
+        """(cells [n] int32 device, offsets [C+1] int32 device): the cells with grid >= 0 (above=False) or
+        grid > 0 (above=True) in ascending order, cascade c's at cells[offsets[c]:offsets[c+1]]."""
+        L = _lib.lib()
+        dev = self.sigma_net.device
+        C, H3 = self.cascade, self.grid_size ** 3
+        cells = torch.empty(C * H3, dtype=torch.int32, device=dev)
+        offsets = torch.empty(C + 1, dtype=torch.int32, device=dev)
+        wbytes = L.nvsf_grid_cell_list_workspace_bytes(C * H3)
+        ws = torch.empty(wbytes, dtype=torch.uint8, device=dev)
+        check(L.nvsf_grid_cell_list(ptr(st["density_grid"]), C, H3, int(above), ptr(cells), ptr(offsets), ptr(ws),
+                                    wbytes, stream_ptr()), "grid_cell_list")
+        return cells, offsets
+
+    def _partial_draws(self, st, seed):
+        """The C*H^3/2 cells of a partial update (nvsf_grid_draws); no host read."""
+        L = _lib.lib()
+        C, H3 = self.cascade, self.grid_size ** 3
+        occupied, offsets = self._cell_list(st, True)
+        cells = torch.empty(C * (H3 // 2), dtype=torch.int32, device=occupied.device)
+        check(L.nvsf_grid_draws(C, H3, int(seed) & (2 ** 64 - 1), st["iter_density"], ptr(occupied), ptr(offsets),
+                                ptr(cells), stream_ptr()), "grid_draws")
+        return cells
+
+    def _refresh_trainable(self, st):
+        """Rebuild the list of trainable cells (grid >= 0) after marks change; one host read of its length.
+        No marked cell: no list, and the full update takes the all-cells path."""
+        cells, offsets = self._cell_list(st, False)
+        k = int(offsets[-1])
+        st["trainable"] = cells[:k] if k < cells.shape[0] else None
+
+    @torch.no_grad()
+    @_lib.device_guard
+    @_lib.with_options
+    def mark_untrained_grid(self, camera_poses=None, intrinsics=None, H=None, W=None, lidar_poses=None,
+                            intrinsics_lidar=None, intrinsics_hoz_lidar=None, cal_lidar_color=False):
+        """torch-ngp's mark_untrained_grid: cells of the occupancy grid of the modality `cal_lidar_color`
+        whose centre no given sensor pose sees (DESIGN.md §3.5: the image frustum of a pinhole camera, the
+        elevation band, range and azimuth wedge of a LiDAR, each widened by two half-cells) get grid = -1
+        and are never occupied; updates skip them.  camera_poses [B,4,4] cam2world with intrinsics (3x3
+        pinhole matrix) and the image size H x W; lidar_poses [B,4,4] lidar2world with intrinsics_lidar =
+        (fov_up, fov) and intrinsics_hoz_lidar = (., fov_hoz) in degrees, range [min_near_lidar,
+        lidar_max_depth].  Either group may be omitted, not both.  Calls accumulate: the marks are those
+        of the union of every pose given so far (a cell seen by a later call is restored to 0).
+        Returns the number of marked cells as a device scalar."""
+        if camera_poses is None and lidar_poses is None:
+            raise _lib.NvsfError("mark_untrained_grid: give camera_poses and / or lidar_poses")
+        L = _lib.lib()
+        lidar = bool(cal_lidar_color)
+        st = self._grid_state(lidar)
+        dev = self.sigma_net.device
+        C, Hg = self.cascade, self.grid_size
+        n = C * Hg ** 3
+        covered = torch.zeros(n // 8, dtype=torch.uint8, device=dev)
+        if st.get("trainable") is not None:  # earlier marks: covered so far == grid >= 0 (marks hold -1)
+            check(L.nvsf_packbits(ptr(st["density_grid"]), n // 8, -0.5, ptr(covered), stream_ptr()), "packbits")
+
+        def poses_of(p, what):
+            p = torch.as_tensor(p).detach().to(device=dev, dtype=torch.float32).contiguous()
+            if p.dim() == 2:
+                p = p.unsqueeze(0)
+            if p.dim() != 3 or p.shape[1:] != (4, 4):
+                raise _lib.NvsfError(f"mark_untrained_grid: {what} must be [B,4,4], got {tuple(p.shape)}")
+            return p
+
+        if camera_poses is not None:
+            if intrinsics is None or H is None or W is None:
+                raise _lib.NvsfError("mark_untrained_grid: camera_poses need intrinsics, H and W")
+            p = poses_of(camera_poses, "camera_poses")
+            K = torch.as_tensor(intrinsics, dtype=torch.float64).cpu()
+            fx, fy, cx, cy = float(K[0, 0]), float(K[1, 1]), float(K[0, 2]), float(K[1, 2])
+            check(L.nvsf_grid_coverage_camera(C, Hg, self.bound, ptr(p), p.shape[0], fx, fy, cx, cy, int(H), int(W),
+                                              ptr(covered), stream_ptr()), "grid_coverage_camera")
+        if lidar_poses is not None:
+            if intrinsics_lidar is None or intrinsics_hoz_lidar is None:
+                raise _lib.NvsfError("mark_untrained_grid: lidar_poses need intrinsics_lidar and intrinsics_hoz_lidar")
+            p = poses_of(lidar_poses, "lidar_poses")
+            check(L.nvsf_grid_coverage_lidar(C, Hg, self.bound, ptr(p), p.shape[0], float(intrinsics_lidar[0]),
+                                             float(intrinsics_lidar[1]), float(intrinsics_hoz_lidar[1]),
+                                             self.min_near_lidar, self.lidar_max_depth, ptr(covered), stream_ptr()),
+                  "grid_coverage_lidar")
+        n_marked = torch.empty(1, dtype=torch.int32, device=dev)
+        check(L.nvsf_grid_apply_marks(ptr(st["density_grid"]), ptr(st["density_bitfield"]), ptr(covered), n,
+                                      ptr(n_marked), stream_ptr()), "grid_apply_marks")
+        self._refresh_trainable(st)
+        return n_marked[0]
+
+    def occupancy_state_dict(self):
+        """The occupancy grids, apart from state_dict(): {"lidar" | "camera": {density_grid (with its -1 marks),
+        density_bitfield, stats, iter_density}} for each modality that has a grid."""
+        names = {True: "lidar", False: "camera"}
+        return {names[k]: dict(density_grid=v["density_grid"].clone(), density_bitfield=v["density_bitfield"].clone(),
+                               stats=v["stats"].clone(), iter_density=int(v["iter_density"]))
+                for k, v in getattr(self, "_grid", {}).items()}
+
+    @torch.no_grad()
+    @_lib.device_guard
+    @_lib.with_options
+    def load_occupancy_state_dict(self, sd):
+        """Load what occupancy_state_dict() returned (CPU or GPU tensors) and rebuild the trainable-cell list."""
+        C, H3 = self.cascade, self.grid_size ** 3
+        n = C * H3
+        for name, v in sd.items():
+            if name not in ("lidar", "camera"):
+                raise _lib.NvsfError(f"load_occupancy_state_dict: unknown modality {name!r}")
+            g, b, s = v["density_grid"], v["density_bitfield"], v["stats"]
+            if g.numel() != n or b.numel() != n // 8 or b.dtype != torch.uint8 or s.numel() != 2:
+                raise _lib.NvsfError(f"load_occupancy_state_dict: {name} grid has {g.numel()} cells / "
+                                     f"{b.numel()} bitfield bytes, this model has C*H^3 = {n} / {n // 8}")
+            st = self._grid_state(name == "lidar")
+            st["density_grid"].view(-1).copy_(g.reshape(-1))
+            st["density_bitfield"].copy_(b.reshape(-1))
+            st["stats"].copy_(s.reshape(-1))
+            st["iter_density"] = int(v["iter_density"])
+            self._refresh_trainable(st)
 
     @torch.no_grad()
     @_lib.device_guard
