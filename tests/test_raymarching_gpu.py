@@ -6,6 +6,7 @@ a build of it (oracle/build_ref.sh).
 Bar: bit-exact for sample ids/offsets/counts, positions, deltas, near/far, Morton codes and
 bitfields; 1e-5 relative for compositing against the oracle (the oracle's exp2f is not the
 GPU's ex2.approx), bit-exact against the reference extension."""
+import contextlib
 import os
 
 import numpy as np
@@ -27,6 +28,22 @@ def dev(a):
 
 def host(t):
     return t.detach().cpu().numpy()
+
+
+@contextlib.contextmanager
+def options(pkg, overrides):
+    """Set library options ({name: value}) for the body and restore the previous values, also when it fails.  Set
+    directly rather than through option_scope: its lock would stall autograd's backward thread, which enters the
+    library through the same lock while the test thread waits in .backward()."""
+    L = pkg._lib.lib()
+    saved = [(k.encode(), L.nvsf_get_option(k.encode())) for k in overrides]
+    try:
+        for k, v in overrides.items():
+            assert L.nvsf_set_option(k.encode(), int(v)) == 0, f"set_option({k}={v})"
+        yield
+    finally:
+        for k, v in reversed(saved):
+            L.nvsf_set_option(k, v)
 
 
 def rel_close(a, b, rtol=1e-5, atol=1e-7, what=""):
@@ -325,9 +342,17 @@ def test_composite_rays_train_properties_full_frame(pkg):
 
 
 # ------------------------------------------------------------------ inference pair
-@pytest.mark.parametrize("fill,n_step_cap", [("shell", 8), ("full", 40), ("random5", 1)])
-def test_inference_loop_matches_oracle(pkg, oracle, ref_ext, fill, n_step_cap):
-    """torch-ngp style run_cuda loop: march_rays -> field -> composite_rays -> compaction."""
+@pytest.mark.parametrize("fill,n_step_cap,march_mode", [
+    pytest.param(f, s, mode, id=f"{f}-{s}" + ("" if mode == 1 else f"-march_mode{mode}"))
+    for mode in (1, 0) for f, s in [("shell", 8), ("full", 40), ("random5", 1)]])
+def test_inference_loop_matches_oracle(pkg, oracle, ref_ext, fill, n_step_cap, march_mode):
+    """torch-ngp style run_cuda loop: march_rays -> field -> composite_rays -> compaction, under the
+    warp-cooperative (march_mode 1, default) and the serial (0) inference marcher."""
+    with options(pkg, {"march_mode": march_mode}):
+        _inference_loop(pkg, oracle, ref_ext, fill, n_step_cap)
+
+
+def _inference_loop(pkg, oracle, ref_ext, fill, n_step_cap):
     rm = pkg.raymarching
     N = 3000
     o, d, nears, fars, _ = cases.march_inputs("lidar", N, seed=31, perturb=False)
@@ -427,8 +452,19 @@ def test_operators_match_reference_golden(pkg, gold):
     assert_bits_equal(host(rm.packbits(dev(g["pb_grid"]), 0.25)), g["pb_bits"], "packbits")
 
 
-@pytest.mark.parametrize("ci", [0, 1, 2, 3])
-def test_march_and_composite_train_match_reference_golden(pkg, gold, ci):
+# the defaults (march_mode 1, composite_mode 2, composite_bwd_mode 2) and every other kernel of the three options
+GOLD_MODES = {"serial-tile": dict(march_mode=0, composite_mode=0, composite_bwd_mode=0),
+              "coop-hybrid": dict(march_mode=1, composite_mode=1, composite_bwd_mode=1)}
+
+
+@pytest.mark.parametrize("ci,modes", [pytest.param(ci, {}, id=str(ci)) for ci in range(4)] +
+                         [pytest.param(ci, m, id=f"{ci}-{name}") for name, m in GOLD_MODES.items() for ci in range(4)])
+def test_march_and_composite_train_match_reference_golden(pkg, gold, ci, modes):
+    with options(pkg, modes):
+        _march_and_composite_train_golden(pkg, gold, ci)
+
+
+def _march_and_composite_train_golden(pkg, gold, ci):
     rm = pkg.raymarching
     p = f"mt{ci}_"
     _, N, max_steps, perturb, m = gold[p + "meta"].tolist()
@@ -451,6 +487,16 @@ def test_march_and_composite_train_match_reference_golden(pkg, gold, ci):
 
 
 def test_inference_step_matches_reference_golden(pkg, gold):
+    _inference_step_golden(pkg, gold)
+
+
+def test_inference_step_matches_reference_golden_serial_marcher(pkg, gold):
+    """The same stored step under march_mode 0: the serial inference marcher must give the reference's bits too."""
+    with options(pkg, {"march_mode": 0}):
+        _inference_step_golden(pkg, gold)
+
+
+def _inference_step_golden(pkg, gold):
     rm = pkg.raymarching
     g = gold
     n_alive, n_step = g["inf_meta"].tolist()
